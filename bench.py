@@ -59,6 +59,11 @@ WORKLOADS = {
     'zoom52': (1024, 'BASELINE configs[4]'),
 }
 
+# --dump-outputs: rays sampled from the last timed step (9 float64 records + status + fail_surf
+# = 88 B a ray, 23 MB at 2^18 rays)
+DUMP_MAX_RAYS = 1 << 18
+DUMP_SEED = 20261017
+
 
 def parse():
     ap = argparse.ArgumentParser()
@@ -74,7 +79,12 @@ def parse():
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--gather-every', type=int, default=8,
                     help='multi-GPU: steps whose spot sums share one all-gather (1 = a collective per step)')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write the results of the last timed step to DIR/<name>.npy (rank 0; a fixed '
+                         'seeded sample of at most %d rays, float64)' % DUMP_MAX_RAYS)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     args.baseline_num = WORKLOADS[args.model][0]
     if args.num is None:
         args.num = args.baseline_num
@@ -392,6 +402,26 @@ def config_dict(args, opm, grid, world):
                   f'{n_rays*80/1e6:.0f} MB of results per grid (L2: 126 MB)'}
 
 
+def dump_outputs(out_dir, res, first_ray):
+    """Write what the timed step returned to its caller -- the per-ray records of ``res`` and
+    the per-(field, wvl) spot sums -- as float64 .npy files under ``out_dir``.  Grids of more
+    than DUMP_MAX_RAYS rays are sampled at ray indices drawn once from a fixed seed, so two
+    builds run with the same arguments write comparable files; ``ray_index.npy`` holds the
+    sampled rays' indices in the whole grid."""
+    os.makedirs(out_dir, exist_ok=True)
+    n = res.n
+    if n > DUMP_MAX_RAYS:
+        idx = np.sort(np.random.default_rng(DUMP_SEED).choice(n, DUMP_MAX_RAYS, replace=False))
+    else:
+        idx = np.arange(n)
+    arrays = {'ray_index': first_ray + idx}
+    for k in ('p', 'd', 'op', 'abr', 'status', 'fail_surf'):
+        arrays[k] = getattr(res, k).cpu().numpy()[..., idx]
+    arrays['spot_sums'] = res.summary.cpu().numpy()
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + '.npy'), np.ascontiguousarray(a, dtype=np.float64))
+
+
 # ----------------------------------------------------------------- B200 arm
 def kernel_name(tab_descs, lean_ok=True):
     poly = any(d.profile > 1 for d in tab_descs)
@@ -559,6 +589,8 @@ def run_b200(args):
         last = combined.reshape(-1, grid.n_tiles, E.RT_SUMMARY_DOUBLES)[-1]
         gather_ok = bool(int(last[:, 0:5].sum().item()) == n_job)
     dev_ms = e_first.elapsed_time(e_last)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, res, first)
     t = torch.tensor([dev_ms, wall*1e3, kern_ms], dtype=torch.float64, device=dev)
     tmin = t.clone()
     if world > 1:

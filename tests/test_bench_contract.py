@@ -65,6 +65,31 @@ def test_b200_arm_line_on_the_dry_run_engine():
         assert line['parity_vs_reference']['bit_identical_p_d_op'] is True
 
 
+def test_b200_arm_dumps_the_last_step_on_the_dry_run_engine(tmp_path):
+    """--dump-outputs DIR: the last timed step's records as float64 .npy files, the same from
+    run to run with the same arguments."""
+    import numpy as np
+    runs = []
+    for k in range(2):
+        out = tmp_path / str(k)
+        p = subprocess.run([sys.executable, os.path.join(ROOT, 'tests', 'dry_bench.py'), '--steps', '2', '--warmup',
+                            '1', '--num', '24', '--no-e2e', '--no-cpu-baseline', '--dump-outputs', str(out)],
+                           capture_output=True, text=True, timeout=900, cwd=ROOT)
+        assert p.returncode == 0, p.stderr[-3000:]
+        assert json.loads(p.stdout.strip().splitlines()[-1])['steps'] == 2
+        runs.append({f.name: np.load(f) for f in sorted(out.iterdir())})
+    a, b = runs
+    assert set(a) == {'ray_index.npy', 'p.npy', 'd.npy', 'op.npy', 'abr.npy', 'status.npy', 'fail_surf.npy',
+                      'spot_sums.npy'}
+    n = 3*3*24*24
+    assert a['p.npy'].shape == (3, n) and a['abr.npy'].shape == (2, n) and a['status.npy'].shape == (n,)
+    assert np.array_equal(a['ray_index.npy'], np.arange(n))
+    assert sum(v.nbytes for v in a.values()) <= 64 << 20
+    for k in a:
+        assert a[k].dtype == np.float64 and np.array_equal(a[k], b[k], equal_nan=True), k
+    assert 0 < (a['status.npy'] == 0).sum() < n
+
+
 def test_b200_arm_two_ranks_on_the_dry_run_engine():
     """world size 2 over gloo (dry-run engine): the eager multi-rank step loop with its asynchronous
     all-gather + combine, max-over-ranks timing and the shard mode's equal-work ranges produce

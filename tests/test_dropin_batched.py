@@ -5,7 +5,8 @@ CPU: rayoptics.raytr.analyses.RayFan / RayList / RayGrid (importable) are run on
 model (oracle/ref_model.py) with their per-ray loops `trace_ray_fan / trace_ray_list /
 trace_ray_grid` rebound to rayoptics_b200.trace's batched stand-ins (oracle-fed through the
 `tracer=` seam) and must reproduce, bit for bit, what the unpatched reference produced
-(tests/golden/vectors/<model>_analyses.npz).  Skipped without /root/reference.
+(tests/golden/vectors/<model>_analyses.npz).  What runs here is the reference's own code, so these
+tests need its source tree (oracle/ref_harness.py, B200RT_REF_SRC) and skip without it.
 """
 import functools
 import os
@@ -18,7 +19,7 @@ from oracle import ref_harness as rh
 from rayoptics_b200 import trace as TR
 from test_trace_drivers import oracle_tracer
 
-pytestmark = pytest.mark.skipif(not rh.available(), reason='/root/reference not present')
+pytestmark = pytest.mark.skipif(not rh.available(), reason='needs the ray-optics source tree (B200RT_REF_SRC)')
 
 
 @pytest.mark.parametrize('name', ['dblgauss', 'rc', 'telecentric', 'fisheye', 'threemir'])

@@ -7,7 +7,7 @@ SOURCE TEXT of `OpticalSpecs.ray_start_from_osp` (opticalspec.py:289-400),
 expose the attributes those functions read (filled from the mirror model).  Their output
 is compared bit for bit with rayoptics_b200/opticalspec.py -- which the oracle and the CUDA
 start-ray kernels are in turn checked against (tests/test_host.py, tests/test_hostsim.py).
-Skipped where /root/reference does not exist.
+The reference's results are stored under tests/golden/reference/ (tests/refdata.py).
 """
 import ast
 import collections
@@ -19,8 +19,7 @@ import pytest
 
 from conftest import load_model
 from oracle import ref_harness as rh
-
-pytestmark = pytest.mark.skipif(not rh.available(), reason='/root/reference not present')
+from refdata import digest, ref  # noqa: F401
 
 ParaxData = collections.namedtuple('ParaxData', ['ax_ray', 'pr_ray', 'fod'])
 
@@ -95,26 +94,41 @@ class FldShim:
         self.aim_info = f.aim_info
 
 
-@pytest.mark.parametrize('name', ['dblgauss', 'triplet', 'rc', 'cellphone', 'thin_triplet', 'exotic',
-                                  'relay_na', 'relay_fno', 'telecentric', 'singlet', 'fisheye', 'threemir'])
-def test_start_rays_equal_the_references_code(name):
+def reference_start_rays(opm, pupils):
+    """per field: the reference's obj_coords, and digest() of its apply_vignetting and
+    ray_start_from_osp for every pupil"""
     methods = reference_methods()
-    opm = load_model(name)
-    osp = opm.optical_spec
     shim = OspShim(opm, methods)
     apply_vig = methods[('Field', 'apply_vignetting')]
+    out = []
+    for f in opm.optical_spec.field_of_view.fields:
+        fs = FldShim(f)
+        p_ref, d_ref = shim.obj_coords(fs)
+        rays = []
+        for pupil in pupils:
+            v_ref = apply_vig(fs, np.array(pupil))
+            pt_ref, dir_ref = shim.ray_start_from_osp(v_ref, fs, 'rel pupil')
+            rays.append((v_ref, pt_ref, dir_ref))
+        out.append((p_ref, d_ref, digest(rays)))
+    return out
+
+
+@pytest.mark.parametrize('name', ['dblgauss', 'triplet', 'rc', 'cellphone', 'thin_triplet', 'exotic',
+                                  'relay_na', 'relay_fno', 'telecentric', 'singlet', 'fisheye', 'threemir'])
+def test_start_rays_equal_the_references_code(name, ref):
+    opm = load_model(name)
+    osp = opm.optical_spec
     rng = np.random.default_rng(4)
     pupils = [np.array(p) for p in ([0., 0.], [0., 1.], [1., 0.], [-1., 0.], [0., -1.])] + \
         [rng.uniform(-1, 1, 2) for _ in range(40)]
-    for f in osp.field_of_view.fields:
-        fs = FldShim(f)
-        p_ref, d_ref = shim.obj_coords(fs)
+    want = ref(lambda: reference_start_rays(opm, pupils))
+    assert len(want) == len(osp.field_of_view.fields)
+    for f, (p_ref, d_ref, rays_ref) in zip(osp.field_of_view.fields, want):
         p_own, d_own = osp.obj_coords(f)
         assert np.array_equal(p_ref, p_own) and np.array_equal(d_ref, d_own)
+        rays = []
         for pupil in pupils:
-            v_ref = apply_vig(fs, np.array(pupil))
             v_own = f.apply_vignetting(np.array(pupil))
-            assert np.array_equal(v_ref, v_own)
-            pt_ref, dir_ref = shim.ray_start_from_osp(v_ref, fs, 'rel pupil')
             pt_own, dir_own = osp.ray_start_from_osp(v_own, f, 'rel pupil')
-            assert np.array_equal(pt_ref, pt_own) and np.array_equal(dir_ref, dir_own)
+            rays.append((v_own, pt_own, dir_own))
+        assert digest(rays) == rays_ref

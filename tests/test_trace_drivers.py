@@ -4,7 +4,8 @@ seq/sequential.py:1006-1120, raytr/analyses.py:46-118).
 
 CPU: the `tracer=` seam is fed by the oracle, the expected values come from the
 reference's own trace_raw on start rays built by opticalspec.ray_start_from_osp
-(skipped without /root/reference) and from the golden OPD vectors.  The GPU run of the
+(stored under tests/golden/reference/ by tests/refdata.py; whole ray packages as digest())
+and from the golden OPD vectors.  The GPU run of the
 same calls is in tests/test_zz_gpu_additions.py.
 """
 import os
@@ -15,6 +16,7 @@ import pytest
 from conftest import load_model
 from rayoptics_b200 import _abi, engine as E, table as T, trace as TR, waveabr as W
 from rayoptics_b200 import analyses as A
+from refdata import digest, lens_files, ref  # noqa: F401
 
 
 def oracle_tracer(opt_model, table, fld, wvl, px, py, apply_vignetting, trace_kwargs):
@@ -49,21 +51,30 @@ def ref_pkg(opm, fld, wvl, pupil, apply_vignetting=True, **kw):
     return rh.ref_trace(rh.ref_path(sm, wvl), pt0, dir0, wvl, **kw)
 
 
+def ref_pkg_digest(*args, **kw):
+    """ref_pkg with the segments [n_seg, 10] as digest()"""
+    r = ref_pkg(*args, **kw)
+    return dict(r, ray=digest(r['ray']))
+
+
+def pkg_digest(pkg):
+    """digest() of a ray package's segments (p, d, dst, nrml) and optical path"""
+    return digest([[tuple(seg)[:4] for seg in pkg[0]], pkg[1]])
+
+
 def assert_pkg_equals(pkg, ref):
     ray, op, _ = pkg
     assert len(ray) == ref['n_seg']
-    for k, seg in enumerate(ray):
-        assert np.array_equal(seg[0], ref['ray'][k, 0:3]) and np.array_equal(seg[1], ref['ray'][k, 3:6])
-        assert seg[2] == ref['ray'][k, 6] and np.array_equal(seg[3], ref['ray'][k, 7:10])
+    if isinstance(ref['ray'], str):             # stored as digest() of the [n_seg, 10] segments
+        assert digest([np.concatenate([seg[0], seg[1], [seg[2]], seg[3]]) for seg in ray]) == ref['ray']
+    else:
+        for k, seg in enumerate(ray):
+            assert np.array_equal(seg[0], ref['ray'][k, 0:3]) and np.array_equal(seg[1], ref['ray'][k, 3:6])
+            assert seg[2] == ref['ray'][k, 6] and np.array_equal(seg[3], ref['ray'][k, 7:10])
     assert op == ref['op']
 
 
-needs_ref = pytest.mark.skipif(not __import__('oracle.ref_harness', fromlist=['x']).available(),
-                               reason='/root/reference not present')
-
-
-@needs_ref
-def test_trace_fan_and_grid_against_reference_rays():
+def test_trace_fan_and_grid_against_reference_rays(ref):
     opm = load_model('dblgauss')
     osp = opm.optical_spec
     fld, wvl = osp.field_of_view.fields[2], 486.1
@@ -74,7 +85,7 @@ def test_trace_fan_and_grid_against_reference_rays():
     # reference's trace_base vignettes its ndarray argument in place)
     assert [f[0][1] for f in fan] == [fld.apply_vignetting(np.array([0., v]))[1] for v in t]
     for (pupil, pkg), v in zip(fan, t):
-        assert_pkg_equals(pkg, ref_pkg(opm, fld, wvl, [0., v]))
+        assert_pkg_equals(pkg, ref(lambda: ref_pkg_digest(opm, fld, wvl, [0., v])))
     # grid: check_apertures forced on, failed rays -> None entries, x outer / y inner
     grid_def = [np.array([-1., -1.]), np.array([1., 1.]), 7]
     seen = []
@@ -88,11 +99,11 @@ def test_trace_fan_and_grid_against_reference_rays():
     n_ok = 0
     raw = [[xs[i], xs[j]] for i in range(7) for j in range(7)]
     for (pupil, pkg), p_raw in zip(seen, raw):
-        ref = ref_pkg(opm, fld, wvl, p_raw, check_apertures=True)
-        assert (pkg is None) == (ref['status'] != 0)
+        want = ref(lambda: ref_pkg_digest(opm, fld, wvl, p_raw, check_apertures=True))
+        assert (pkg is None) == (want['status'] != 0)
         if pkg is not None:
             n_ok += 1
-            assert_pkg_equals(pkg, ref)
+            assert_pkg_equals(pkg, want)
     assert 0 < n_ok < 49 and g.shape == (n_ok,)
     g2 = TR.trace_grid(opm, grid_def, fld, wvl, 0.0, tracer=oracle_tracer)
     assert g2.shape[:2] == (7, 7)
@@ -154,8 +165,7 @@ def oracle_bundle_tracer(opt_model, table, p0, d0, wvl_idx, trace_kwargs):
                                   want_full=True, wvls=wvls)
 
 
-@needs_ref
-def test_trace_list_of_rays():
+def test_trace_list_of_rays(ref):
     from conftest import load_vectors
     from oracle import ref_harness as rh
     opm = load_model('triplet')
@@ -168,14 +178,17 @@ def test_trace_list_of_rays():
                                check_apertures=case['check_apertures'])
     assert len(out) == len(rays)
     n_err = 0
+    def ref_trace(pt0, dir0, wvl):
+        r = rh.ref_trace(rh.ref_path(sm, wvl), pt0, dir0, wvl, **case)
+        return dict(r, ray=digest(r['ray']))
     for (pt0, dir0, wvl), item in zip(rays, out):
-        ref = rh.ref_trace(rh.ref_path(sm, wvl), pt0, dir0, wvl, **case)
-        if ref['status'] == 0:
-            assert_pkg_equals(item, ref)
+        want = ref(lambda: ref_trace(pt0, dir0, wvl))
+        if want['status'] == 0:
+            assert_pkg_equals(item, want)
         else:
             n_err += 1
             ray, err = item
-            assert err.surf == ref['fail_surf'] and len(err.ray_pkg[0]) == ref['n_seg']
+            assert err.surf == want['fail_surf'] and len(err.ray_pkg[0]) == want['n_seg']
     last = A.trace_list_of_rays(opm, rays, output_filter='last', tracer=oracle_bundle_tracer,
                                 check_apertures=case['check_apertures'])
     assert len(last) == len(rays) - n_err and len(last[0]) == 3 and len(last[0][0]) == 4
@@ -287,10 +300,9 @@ def test_trace_ray_and_boundary_rays():
     assert hts[0] == pytest.approx(opm.seq_model.ifcs[2].max_aperture, rel=1e-6)
 
 
-@needs_ref
-def test_iterate_ray_is_the_references():
+def test_iterate_ray_is_the_references(ref):
     """vigcalc.iterate_ray against the reference's iterate_ray, whose source text is executed
-    from /root/reference (its module cannot be imported: opticalglass is absent) on the
+    from the reference tree (its module cannot be imported: opticalglass is absent) on the
     reference's own trace_raw."""
     import ast
     import logging
@@ -298,10 +310,11 @@ def test_iterate_ray_is_the_references():
     from scipy.optimize import newton, fsolve
     from oracle import ref_harness as rh
     from rayoptics_b200 import vigcalc as V
-    R = rh.ref()
-    src = open('/root/reference/src/rayoptics/raytr/trace.py').read()
-    fn = [n for n in ast.parse(src).body if isinstance(n, ast.FunctionDef) and n.name == 'iterate_ray'][0]
-    for name, fi in (('triplet', 1), ('thin_triplet', 1), ('exotic', 2)):
+
+    def reference_iterate_ray(name, fi):
+        R = rh.ref()
+        src = open(os.path.join(rh.REF_SRC, 'rayoptics', 'raytr', 'trace.py')).read()
+        fn = [n for n in ast.parse(src).body if isinstance(n, ast.FunctionDef) and n.name == 'iterate_ray'][0]
         opm = load_model(name)
         sm, osp = opm.seq_model, opm.optical_spec
         paths = {}
@@ -332,8 +345,15 @@ def test_iterate_ray_is_the_references():
                   warnings=warnings, logger=logging.getLogger('ref'), mc=type('mc', (), {'p': 0}))
         exec(ast.get_source_segment(src, fn), ns)
         fld = osp.field_of_view.fields[fi]
+        want, _ = ns['iterate_ray'](Opm(), sm.stop_surface, np.array([0., 0.]), fld, sm.central_wavelength())
+        return want
+
+    for name, fi in (('triplet', 1), ('thin_triplet', 1), ('exotic', 2)):
+        opm = load_model(name)
+        sm, osp = opm.seq_model, opm.optical_spec
+        fld = osp.field_of_view.fields[fi]
         wvl = sm.central_wavelength()
-        want, _ = ns['iterate_ray'](Opm(), sm.stop_surface, np.array([0., 0.]), fld, wvl)
+        want = ref(lambda: reference_iterate_ray(name, fi))
 
         def our_trace(seq_model, pt0, dir0, wvl, **kw):       # engine stand-in: the oracle
             r = oracle_bundle_tracer(opm, None, np.array(pt0, dtype=float).reshape(3, 1),
@@ -352,55 +372,20 @@ def test_iterate_ray_is_the_references():
         assert np.array_equal(got, want), (name, got, want)
 
 
-@needs_ref
 @pytest.mark.parametrize('name,fi,wvl', [('dblgauss', 2, 486.1), ('rc', 3, 550.0), ('thin_triplet', 1, 587.6)])
-def test_drivers_against_the_references_drivers(name, fi, wvl):
+def test_drivers_against_the_references_drivers(name, fi, wvl, ref):
     """trace_fan / trace_grid / trace_base / setup_pupil_coords of rayoptics_b200.trace (oracle-fed)
     against the REFERENCE's own functions of the same names (rayoptics.raytr.trace is importable)
-    running on a hybrid model with the reference's trace_raw (oracle/ref_model.py)."""
-    from oracle import ref_model
-    RT, RA = ref_model.modules()
+    running on a hybrid model with the reference's trace_raw (oracle/ref_model.py).  The reference
+    re-aims the field's chief ray and keeps the aim point on the field; each call here starts from
+    the aim point the reference's call of the same name left."""
     opm = load_model(name)
     if wvl not in opm.seq_model.wvlns:
         wvl = opm.seq_model.central_wavelength()
-    H = ref_model.HybridModel(opm)
     fld = opm.optical_spec.field_of_view.fields[fi]
-
-    def same_pkg(a, b):
-        assert len(a[0]) == len(b[0]) and a[1] == b[1]
-        for sa, sb in zip(a[0], b[0]):
-            assert np.array_equal(sa[0], sb[0]) and np.array_equal(sa[1], sb[1])
-            assert sa[2] == sb[2] and np.array_equal(sa[3], sb[3])
-
-    # chief ray + reference sphere
-    rs_ref, cr_ref = RT.setup_pupil_coords(H, fld, wvl, 0.0)
-    rs_own, cr_own = TR.setup_pupil_coords(opm, fld, wvl, 0.0, tracer=oracle_tracer)
-    same_pkg(cr_own[0], cr_ref[0])
-    assert np.array_equal(rs_own[0], rs_ref[0]) and np.array_equal(rs_own[1], rs_ref[1])
-    assert rs_own[2] == rs_ref[2]
-    for a, b in zip(cr_own[1][:3], cr_ref[1][:3]):
-        assert np.array_equal(a, b)
-    # fan with an OPD callback evaluated by the reference's waveabr on both sides
-    import importlib
-    WR = importlib.import_module('rayoptics.raytr.waveabr')
-    fod = opm.optical_spec.fod
-
-    def opd_ref(p, pkg):
-        return WR.wave_abr_full_calc(fod, fld, wvl, 0.0, pkg, cr_ref, rs_ref)
-
-    def opd_own(p, pkg):
-        return W.wave_abr_full_calc(fod, fld, wvl, 0.0, pkg, cr_own, rs_own)
-
     fan_def = lambda: [np.array([0., -1.]), np.array([0., 1.]), 11]      # noqa: E731
-    f_ref = RT.trace_fan(H, fan_def(), fld, wvl, 0.0, img_filter=opd_ref)
-    f_own = TR.trace_fan(opm, fan_def(), fld, wvl, 0.0, img_filter=opd_own, tracer=oracle_tracer)
-    assert len(f_ref) == len(f_own) > 3
-    for (pa, va), (pb, vb) in zip(f_own, f_ref):
-        assert np.array_equal(pa, pb) and va == vb
-    # grid with a callback (the reference's own np.array(grid) cannot hold raw packages under
-    # numpy >= 1.24); blocked rays reach the callback as None
     grid_def = lambda: [np.array([-1., -1.]), np.array([1., 1.]), 7]     # noqa: E731
-    seen_ref, seen_own = [], []
+    pupils = ([0.3, -0.2], [0., 1.4])
 
     def cb(store):
         def f(p, pkg):
@@ -408,28 +393,83 @@ def test_drivers_against_the_references_drivers(name, fi, wvl):
             return np.array([p[0], p[1], np.nan if pkg is None else pkg[1]])
         return f
 
-    g_ref = RT.trace_grid(H, grid_def(), fld, wvl, 0.0, form='grid', img_filter=cb(seen_ref))
+    def reference_side():
+        import importlib
+        from oracle import ref_model
+        RT, RA = ref_model.modules()
+        a = load_model(name)
+        H = ref_model.HybridModel(a)
+        fa = a.optical_spec.field_of_view.fields[fi]
+        aims = []                               # fa.aim_info after each stage
+
+        def aim():
+            aims.append(None if fa.aim_info is None else np.array(fa.aim_info, dtype=float))
+        # chief ray + reference sphere
+        rs_ref, cr_ref = RT.setup_pupil_coords(H, fa, wvl, 0.0)
+        aim()
+        # fan with an OPD callback evaluated by the reference's waveabr
+        WR = importlib.import_module('rayoptics.raytr.waveabr')
+        fod = a.optical_spec.fod
+        f_ref = RT.trace_fan(H, fan_def(), fa, wvl, 0.0,
+                             img_filter=lambda p, pkg: WR.wave_abr_full_calc(fod, fa, wvl, 0.0, pkg, cr_ref, rs_ref))
+        aim()
+        # grid with a callback (the reference's own np.array(grid) cannot hold raw packages under
+        # numpy >= 1.24); blocked rays reach the callback as None
+        seen = []
+        g_ref = RT.trace_grid(H, grid_def(), fa, wvl, 0.0, form='grid', img_filter=cb(seen))
+        aim()
+        singles = []
+        for pupil in pupils:
+            try:
+                singles.append(pkg_digest(RT.trace_base(H, np.array(pupil), fa, wvl, check_apertures=True)))
+            except R_TraceError() as e:
+                singles.append((type(e).__name__, e.surf))
+            aim()
+        return {'aims': aims, 'cr_pkg': pkg_digest(cr_ref[0]), 'cr': list(cr_ref[1][:3]), 'rs': list(rs_ref[:3]),
+                'fan': f_ref, 'grid': g_ref, 'seen': [None if p is None else pkg_digest(p) for p in seen],
+                'singles': singles}
+    want = ref(reference_side)
+    aims = iter(want['aims'])
+
+    # chief ray + reference sphere
+    fld.aim_info = next(aims)
+    rs_own, cr_own = TR.setup_pupil_coords(opm, fld, wvl, 0.0, tracer=oracle_tracer)
+    assert pkg_digest(cr_own[0]) == want['cr_pkg']
+    assert np.array_equal(rs_own[0], want['rs'][0]) and np.array_equal(rs_own[1], want['rs'][1])
+    assert rs_own[2] == want['rs'][2]
+    for a, b in zip(cr_own[1][:3], want['cr']):
+        assert np.array_equal(a, b)
+    # fan with an OPD callback evaluated by this package's waveabr
+    fod = opm.optical_spec.fod
+
+    def opd_own(p, pkg):
+        return W.wave_abr_full_calc(fod, fld, wvl, 0.0, pkg, cr_own, rs_own)
+
+    fld.aim_info = next(aims)
+    f_own = TR.trace_fan(opm, fan_def(), fld, wvl, 0.0, img_filter=opd_own, tracer=oracle_tracer)
+    assert len(want['fan']) == len(f_own) > 3
+    for (pa, va), (pb, vb) in zip(f_own, want['fan']):
+        assert np.array_equal(pa, pb) and va == vb
+    seen_own = []
+    fld.aim_info = next(aims)
     g_own = TR.trace_grid(opm, grid_def(), fld, wvl, 0.0, form='grid', img_filter=cb(seen_own),
                           tracer=oracle_tracer)
+    g_ref = want['grid']
     assert g_ref.shape == g_own.shape == (7, 7, 3) and np.array_equal(g_ref, g_own, equal_nan=True)
     assert 0 < np.isnan(g_ref[:, :, 2]).sum() < 49
-    for a, b in zip(seen_own, seen_ref):
-        assert (a is None) == (b is None)
-        if a is not None:
-            same_pkg(a, b)
+    assert [None if p is None else pkg_digest(p) for p in seen_own] == want['seen']
     # single ray, error packaging
-    for pupil in ([0.3, -0.2], [0., 1.4]):
-        try:
-            want = RT.trace_base(H, np.array(pupil), fld, wvl, check_apertures=True)
-        except R_TraceError() as e:
+    for pupil, w in zip(pupils, want['singles']):
+        fld.aim_info = next(aims)
+        if isinstance(w, tuple):                # the reference raised (error class name, surface)
             with pytest.raises(type(TR.trace_pupil_rays(opm, [pupil], fld, wvl, None, 'full',
                                                         tracer=oracle_tracer,
                                                         check_apertures=True)[0].err)) as info:
                 TR.trace_base(opm, np.array(pupil), fld, wvl, tracer=oracle_tracer, check_apertures=True)
-            assert type(info.value).__name__ == type(e).__name__ and info.value.surf == e.surf
+            assert (type(info.value).__name__, info.value.surf) == w
         else:
-            same_pkg(TR.trace_base(opm, np.array(pupil), fld, wvl, tracer=oracle_tracer,
-                                   check_apertures=True), want)
+            assert pkg_digest(TR.trace_base(opm, np.array(pupil), fld, wvl, tracer=oracle_tracer,
+                                            check_apertures=True)) == w
 
 
 def oracle_ray_fn(opm):
@@ -468,134 +508,140 @@ def R_TraceError():
     return rh.ref().traceerror.TraceError
 
 
-@needs_ref
 @pytest.mark.parametrize('name', ['dblgauss', 'triplet'])
-def test_set_vig_and_apertures_equal_the_references(name):
+def test_set_vig_and_apertures_equal_the_references(name, ref):
     """vigcalc.set_clear_apertures_batched and vigcalc.set_vig against the reference's
     rayoptics.raytr.vigcalc run unmodified on the hybrid model (reference trace_raw, scipy
     newton): apertures and vignetting factors bit for bit.  The reference's re-aiming is
     bypassed as in make_golden_analyses.py (placeholder chief_ray)."""
-    import importlib
-    from oracle import ref_model
     from rayoptics_b200 import vigcalc as V
-    ref_model.modules()
-    RV = importlib.import_module('rayoptics.raytr.vigcalc')
-    a, b = load_model(name), load_model(name)
-    H = ref_model.HybridModel(a)
-    for f in a.optical_spec.field_of_view.fields:
-        f.chief_ray = ((None, None, -1.0), None)
-    RV.set_clear_apertures(H)
+
+    def reference_side():
+        import importlib
+        from oracle import ref_model
+        ref_model.modules()
+        RV = importlib.import_module('rayoptics.raytr.vigcalc')
+        a = load_model(name)
+        H = ref_model.HybridModel(a)
+        for f in a.optical_spec.field_of_view.fields:
+            f.chief_ray = ((None, None, -1.0), None)
+        RV.set_clear_apertures(H)
+        ap = [ifc.max_aperture for ifc in H.seq_model.ifcs]
+        for f in a.optical_spec.field_of_view.fields:     # vignetting from those apertures, from zero
+            f.vux = f.vlx = f.vuy = f.vly = 0.0
+            f.chief_ray = ((None, None, -1.0), None)
+        RV.set_vig(H)
+        return ap, [(f.vux, f.vlx, f.vuy, f.vly) for f in a.optical_spec.field_of_view.fields]
+    ref_ap, ref_vig = ref(reference_side)
+    b = load_model(name)
     V.set_clear_apertures_batched(b, oracle_bundle_fn(b))
-    ref_ap = [ifc.max_aperture for ifc in H.seq_model.ifcs]
     own_ap = [ifc.max_aperture for ifc in b.seq_model.ifcs]
     assert ref_ap[1:] == own_ap[1:]
     # vignetting from those apertures (both sides start from zero vignetting)
-    for m in (a, b):
-        for f in m.optical_spec.field_of_view.fields:
-            f.vux = f.vlx = f.vuy = f.vly = 0.0
-    for f in a.optical_spec.field_of_view.fields:
-        f.chief_ray = ((None, None, -1.0), None)
-    RV.set_vig(H)
+    for f in b.optical_spec.field_of_view.fields:
+        f.vux = f.vlx = f.vuy = f.vly = 0.0
     V.set_vig(b, tracer=oracle_tracer)
-    for fa, fb in zip(a.optical_spec.field_of_view.fields, b.optical_spec.field_of_view.fields):
-        assert (fa.vux, fa.vlx, fa.vuy, fa.vly) == (fb.vux, fb.vlx, fb.vuy, fb.vly)
+    assert ref_vig == [(f.vux, f.vlx, f.vuy, f.vly) for f in b.optical_spec.field_of_view.fields]
 
 
-@needs_ref
-def test_sequential_model_methods_equal_the_references():
+def test_sequential_model_methods_equal_the_references(ref):
     """SequentialModel.trace_fan / trace_grid / trace_wavefront (seq/sequential.py:1006-1119): the
     reference's METHOD TEXT (the module cannot be imported: opticalglass) executed on the hybrid
     model with the reference's trace functions, against the mirror's methods (oracle-fed)."""
-    import ast
-    import importlib
-    from oracle import ref_model
-    RT, RA = ref_model.modules()
-    src = open('/root/reference/src/rayoptics/seq/sequential.py').read()
-    cls = [n for n in ast.parse(src).body if isinstance(n, ast.ClassDef) and n.name == 'SequentialModel'][0]
-    ns = dict(np=np, trace=RT, waveabr=importlib.import_module('rayoptics.raytr.waveabr'))
-    for fn in cls.body:
-        if isinstance(fn, ast.FunctionDef) and fn.name in ('trace_fan', 'trace_grid', 'trace_wavefront'):
-            exec(ast.get_source_segment(src, fn), ns)
-    a, b = load_model('dblgauss'), load_model('dblgauss')
-    H = ref_model.HybridModel(a)
-    H.seq_model.opt_model = H
-    for f in a.optical_spec.field_of_view.fields:          # no re-aiming by the reference
-        f.chief_ray = ((None, None, -1.0), None)
-
     def y_abr(p, xy, ray_pkg, fld, wvl, foc):
         return ray_pkg[0][-1][0][xy] - fld.ref_sphere[0][xy]
-
-    want = ns['trace_fan'](H.seq_model, y_abr, 2, 1, num_rays=9)
-    got = b.seq_model.trace_fan(y_abr, 2, 1, num_rays=9, tracer=oracle_tracer)
-    assert np.array_equal(want[0], got[0]) and np.array_equal(want[1], got[1]) and want[2] == got[2]
 
     def ht(p, wi, ray_pkg, fld, wvl, foc):
         return None if ray_pkg is None else np.array([p[0], p[1], ray_pkg[0][-1][0][1]])
 
-    want, _ = ns['trace_grid'](H.seq_model, ht, 1, num_rays=6, form='list', append_if_none=False)
+    def reference_side():
+        import ast
+        import importlib
+        from oracle import ref_model, ref_harness as rh
+        RT, RA = ref_model.modules()
+        src = open(os.path.join(rh.REF_SRC, 'rayoptics', 'seq', 'sequential.py')).read()
+        cls = [n for n in ast.parse(src).body if isinstance(n, ast.ClassDef) and n.name == 'SequentialModel'][0]
+        ns = dict(np=np, trace=RT, waveabr=importlib.import_module('rayoptics.raytr.waveabr'))
+        for fn in cls.body:
+            if isinstance(fn, ast.FunctionDef) and fn.name in ('trace_fan', 'trace_grid', 'trace_wavefront'):
+                exec(ast.get_source_segment(src, fn), ns)
+        a = load_model('dblgauss')
+        H = ref_model.HybridModel(a)
+        H.seq_model.opt_model = H
+        for f in a.optical_spec.field_of_view.fields:          # no re-aiming by the reference
+            f.chief_ray = ((None, None, -1.0), None)
+        fan = ns['trace_fan'](H.seq_model, y_abr, 2, 1, num_rays=9)
+        grid, _ = ns['trace_grid'](H.seq_model, ht, 1, num_rays=6, form='list', append_if_none=False)
+        wf = ns['trace_wavefront'](H.seq_model, a.optical_spec.field_of_view.fields[1], 587.6, 0.0, num_rays=8)
+        return fan[:3], [np.array(list(w), dtype=float) for w in grid], wf
+    want_fan, want_grid, want_wf = ref(reference_side)
+    b = load_model('dblgauss')
+    got = b.seq_model.trace_fan(y_abr, 2, 1, num_rays=9, tracer=oracle_tracer)
+    assert np.array_equal(want_fan[0], got[0]) and np.array_equal(want_fan[1], got[1]) and want_fan[2] == got[2]
     got, _ = b.seq_model.trace_grid(ht, 1, num_rays=6, form='list', append_if_none=False,
                                     tracer=oracle_tracer)
-    assert len(want) == len(got) == 3
-    for w, g in zip(want, got):
-        assert np.array_equal(np.array(list(w), dtype=float), np.array(list(g), dtype=float))
-    fa, fb = a.optical_spec.field_of_view.fields[1], b.optical_spec.field_of_view.fields[1]
-    want = ns['trace_wavefront'](H.seq_model, fa, 587.6, 0.0, num_rays=8)
-    got = b.seq_model.trace_wavefront(fb, 587.6, 0.0, num_rays=8, tracer=oracle_tracer)
-    assert np.array_equal(want, got)
+    assert len(want_grid) == len(got) == 3
+    for w, g in zip(want_grid, got):
+        assert np.array_equal(w, np.array(list(g), dtype=float))
+    got = b.seq_model.trace_wavefront(b.optical_spec.field_of_view.fields[1], 587.6, 0.0, num_rays=8,
+                                      tracer=oracle_tracer)
+    assert np.array_equal(want_wf, got)
 
 
-@needs_ref
-def test_find_real_enp_is_the_references():
+def test_find_real_enp_is_the_references(ref):
     """rayoptics_b200/wideangle.py (the wide-angle entrance pupil search) against the reference's
     raytr/wideangle.py find_real_enp run unmodified on the hybrid model: same z_enp, bit for bit,
-    for every field of the fisheye fixture -- from scratch (no aim info) and with the stored value."""
-    import importlib
+    for every field of the fisheye fixture -- from scratch (no aim info) and with the stored value.
+    The reference searches with its own trace_raw, this package's search with the oracle."""
     import warnings
-    from oracle import ref_model, ref_harness as rh
     from rayoptics_b200 import wideangle as W
-    ref_model.modules()
-    RW = importlib.import_module('rayoptics.raytr.wideangle')
-    a, b = load_model('fisheye'), load_model('fisheye')
-    H = ref_model.HybridModel(a)
-    R = rh.ref()
+    b = load_model('fisheye')
+    wvl = b.seq_model.central_wavelength()
+    stored = [f.aim_info for f in b.optical_spec.field_of_view.fields]
+    starts = [(None, s) for s in stored]
 
-    def ref_trace_fn(sm, pt0, dir0, wvl, **kw):
-        kw.setdefault('first_surf', 1)
-        kw.setdefault('last_surf', sm.get_num_surfaces() - 2)
-        return R.raytrace.trace_raw(iter(rh.ref_path(sm, wvl)), np.array(pt0, dtype=float),
-                                    np.array(dir0, dtype=float), wvl, **kw)
-
-    import rayoptics_b200.raytrace as BR
-    wvl = a.seq_model.central_wavelength()
-    stored = [f.aim_info for f in a.optical_spec.field_of_view.fields]
-    for fa, fb, s in zip(a.optical_spec.field_of_view.fields, b.optical_spec.field_of_view.fields, stored):
-        for start in (None, s):
-            fa.aim_info = fb.aim_info = start
+    def reference_side():
+        import importlib
+        from oracle import ref_model, ref_harness as rh
+        ref_model.modules()
+        RW = importlib.import_module('rayoptics.raytr.wideangle')
+        a = load_model('fisheye')
+        H = ref_model.HybridModel(a)
+        out = []
+        for fa, pair in zip(a.optical_spec.field_of_view.fields, starts):
+            for start in pair:
+                fa.aim_info = start
+                with warnings.catch_warnings():
+                    warnings.simplefilter('ignore')
+                    z_ref, rr = RW.find_real_enp(H, a.seq_model.stop_surface, fa, wvl)
+                out.append((z_ref, rr.err is None, len(rr.pkg.ray), rr.pkg.ray[-1][0], rr.pkg.op))
+        fa = a.optical_spec.field_of_view.fields[1]
+        with warnings.catch_warnings():
+            warnings.simplefilter('ignore')
+            cw, rw, _ = RW.find_z_enp(H, a.seq_model.stop_surface, a.optical_spec.fod.enp_dist, fa, wvl)
+        return out, cw
+    want, cw = ref(reference_side)
+    tf = oracle_trace_fn(b)
+    k = 0
+    for fb, pair in zip(b.optical_spec.field_of_view.fields, starts):
+        for start in pair:
+            fb.aim_info = start
             with warnings.catch_warnings():
                 warnings.simplefilter('ignore')
-                z_ref, rr = RW.find_real_enp(H, a.seq_model.stop_surface, fa, wvl)
-                # the mirror's search raises / catches the mirror's TraceError classes: give it a
-                # tracer that translates the reference's exceptions
-                def tf(sm, pt0, dir0, w, **kw):
-                    try:
-                        return ref_trace_fn(sm, pt0, dir0, w, **kw)
-                    except R.traceerror.TraceError as e:
-                        cls = getattr(BR, type(e).__name__)
-                        err = cls.__new__(cls)
-                        err.__dict__.update(e.__dict__)
-                        raise err
                 z_own, rr_own = W.find_real_enp(b, b.seq_model.stop_surface, fb, wvl, trace_fn=tf)
+            z_ref, ok, n_ray, p_last, op = want[k]
+            k += 1
             assert z_own == z_ref
-            assert abs(z_ref - s) < 1e-9
+            assert abs(z_ref - pair[1]) < 1e-9
             # the second return value is the reference's: RayResult of the last ray traced
-            assert (rr_own.err is None) == (rr.err is None) and len(rr_own.pkg.ray) == len(rr.pkg.ray)
-            assert np.array_equal(rr_own.pkg.ray[-1][0], rr.pkg.ray[-1][0]) and rr_own.pkg.op == rr.pkg.op
+            assert (rr_own.err is None) == ok and len(rr_own.pkg.ray) == n_ray
+            assert np.array_equal(rr_own.pkg.ray[-1][0], p_last) and rr_own.pkg.op == op
+    assert k == len(want)
     # the older secant-only search from the paraxial pupil, and the pupil curve across the field
-    fa, fb = a.optical_spec.field_of_view.fields[1], b.optical_spec.field_of_view.fields[1]
-    fod = a.optical_spec.fod
+    fb = b.optical_spec.field_of_view.fields[1]
+    fod = b.optical_spec.fod
     with warnings.catch_warnings():
         warnings.simplefilter('ignore')
-        cw, rw, _ = RW.find_z_enp(H, a.seq_model.stop_surface, fod.enp_dist, fa, wvl)
         cg, rg, res = W.find_z_enp(b, b.seq_model.stop_surface, fod.enp_dist, fb, wvl, trace_fn=tf)
     assert np.array_equal(cw, cg) and res.converged and abs(cg[2] - stored[1]) < 1e-5
     rel = b.optical_spec.field_of_view.is_relative
@@ -628,139 +674,186 @@ def _hybrid_with_powers(opm):
     return H
 
 
-@needs_ref
 @pytest.mark.parametrize('name', ['dblgauss', 'triplet', 'rc', 'evenasph', 'cellphone', 'telecentric'])
-def test_trace_module_call_surface_equals_the_references(name, capsys):
+def test_trace_module_call_surface_equals_the_references(name, capsys, ref):
     """refocus, trace_with_opd, trace_astigmatism(_curve), the Coddington trace, the DataFrame
     listings and the printers of rayoptics.raytr.trace, run by the reference on the hybrid model
     and here on the batched drivers (oracle in the tracer seam): identical numbers / text."""
-    from oracle import ref_model
-    RT, RA = ref_model.modules()
-    a, b = load_model(name), load_model(name)
-    H = _hybrid_with_powers(a)
-    kw = dict(tracer=oracle_tracer)
-    fa, fb = a.optical_spec.field_of_view.fields[-1], b.optical_spec.field_of_view.fields[-1]
-    wvl = a.seq_model.central_wavelength()
-
-    assert RT.refocus(H) == TR.refocus(b, **kw)
-
-    for foc in (0.0, 0.02):
-        want = RT.trace_astigmatism(H, fa, wvl, foc)
-        got = TR.trace_astigmatism(b, fb, wvl, foc, **kw)
-        assert want == got and np.isfinite(got).all()
-    # trace_astigmatism_curve: the reference's loop body (trace.py:812-822) on the reference's
-    # functions (its own Field class needs opticalglass to import, the mirror's Field stands in)
+    import contextlib
+    import io
     from rayoptics_b200.model import Field
-    fov = a.optical_spec.field_of_view
-    fld = Field(fov=fov)
-    sw, tw = [], []
-    for f in np.linspace(0., fov.max_field()[0], num=5):
-        fld.yv = f
-        ref_sphere, cr_pkg = RT.setup_pupil_coords(H, fld, wvl, 0.0)
-        fld.chief_ray, fld.ref_sphere = cr_pkg, ref_sphere
-        s_foc, t_foc = RT.trace_astigmatism(H, fld, wvl, 0.0)
-        sw.append(s_foc)
-        tw.append(t_foc)
+    P1, V1 = np.array([0., 1., 0.]), np.array([0., -0.1, 1.])/np.linalg.norm([0., -0.1, 1.])
+    P2, V2 = np.array([0., -1., 0.]), np.array([0., 0.1, 1.])/np.linalg.norm([0., 0.1, 1.])
+    spherical = name in ('dblgauss', 'triplet', 'telecentric')
+    opd_pupils = ([0., 0.6], [0.4, -0.3])
+
+    def df_values(df):
+        return list(df.index), list(df.columns), digest([[np.asarray(x) for x in df[col]] for col in df.columns])
+
+    def reference_side():
+        from oracle import ref_model
+        RT, RA = ref_model.modules()
+        a = load_model(name)
+        H = _hybrid_with_powers(a)
+        fa = a.optical_spec.field_of_view.fields[-1]
+        wvl = a.seq_model.central_wavelength()
+        out = {'refocus': RT.refocus(H),
+               'astigmatism': [RT.trace_astigmatism(H, fa, wvl, foc) for foc in (0.0, 0.02)]}
+        # trace_astigmatism_curve: the reference's loop body (trace.py:812-822) on the reference's
+        # functions (its own Field class needs opticalglass to import, the mirror's Field stands in)
+        fov = a.optical_spec.field_of_view
+        fld = Field(fov=fov)
+        sw, tw = [], []
+        for f in np.linspace(0., fov.max_field()[0], num=5):
+            fld.yv = f
+            ref_sphere, cr_pkg = RT.setup_pupil_coords(H, fld, wvl, 0.0)
+            fld.chief_ray, fld.ref_sphere = cr_pkg, ref_sphere
+            s_foc, t_foc = RT.trace_astigmatism(H, fld, wvl, 0.0)
+            sw.append(s_foc)
+            tw.append(t_foc)
+        out['curve'] = (sw, tw)
+        # Coddington trace along the chief ray of the outer field
+        pw = RT.trace_ray(H, [0., 0.], fa, wvl)[0]
+        out['chief'] = {'n_seg': len(pw.ray), 'op': pw.op,
+                        'ray': digest(np.array([np.concatenate([s.p, s.d, [s.dst], s.nrml]) for s in pw.ray]))}
+        if spherical:
+            out['coddington'] = [RT.trace_coddington_fan(H, pw, foc=foc) for foc in (None, 0.01)]
+            out['coddington_astigmatism'] = RT.trace_astigmatism_coddington_fan(H, fa, wvl, 0.0)
+        # OPD of single rays (chief ray present on the field: no re-aiming)
+        out['opd'] = []
+        for pupil in opd_pupils:
+            fa.chief_ray = ((None, None, -1.0), None)
+            rw = RT.trace_with_opd(H, list(pupil), fa, wvl, 0.01)
+            out['opd'].append((rw[1], rw[2], rw[3], rw[0][-1][0]))
+        out['all_fields'] = df_values(RT.trace_all_fields(H))
+        out['ray_pkg_index'] = RT.ray_pkg(pw).index.tolist()
+        # printers
+        text = io.StringIO()
+        with contextlib.redirect_stdout(text):
+            RT.list_ray(pw)
+            RT.list_ray((pw, None), tfrms=[(np.identity(3), np.array([0., 0., float(k)])) for k in range(len(pw.ray))],
+                        start=2)
+            RT.list_in_out_dir(list(H.seq_model.path(wvl)), pw.ray)
+        out['printed'] = text.getvalue()
+        out['intersect'] = RT.intersect_2_lines(P1, V1, P2, V2)
+        return out
+    want = ref(reference_side)
+
+    b = load_model(name)
+    kw = dict(tracer=oracle_tracer)
+    fb = b.optical_spec.field_of_view.fields[-1]
+    wvl = b.seq_model.central_wavelength()
+
+    assert want['refocus'] == TR.refocus(b, **kw)
+
+    for w, foc in zip(want['astigmatism'], (0.0, 0.02)):
+        got = TR.trace_astigmatism(b, fb, wvl, foc, **kw)
+        assert w == got and np.isfinite(got).all()
+    fov = b.optical_spec.field_of_view
     fg, sg, tg = TR.trace_astigmatism_curve(b, num_points=5, **kw)
+    sw, tw = want['curve']
     assert list(fg) == list(np.linspace(0., fov.max_field()[0], num=5)) and sw == sg and tw == tg
     assert fov.max_field()[0] > 0 and abs(sg[0] - tg[0]) < 1e-9 < abs(sg[-1] - tg[-1])
 
     # Coddington trace along the chief ray of the outer field
-    pw = RT.trace_ray(H, [0., 0.], fa, wvl)[0]
     pg = TR.trace_ray(b, [0., 0.], fb, wvl, **kw)[0]
-    assert_pkg_equals(pg, {'n_seg': len(pw.ray), 'op': pw.op,
-                           'ray': np.array([np.concatenate([s.p, s.d, [s.dst], s.nrml]) for s in pw.ray])})
-    if name in ('dblgauss', 'triplet', 'telecentric'):    # spherical surfaces only
-        for foc in (None, 0.01):
-            want = RT.trace_coddington_fan(H, pw, foc=foc)
+    assert_pkg_equals(pg, want['chief'])
+    if spherical:                               # spherical surfaces only
+        for w, foc in zip(want['coddington'], (None, 0.01)):
             got = TR.trace_coddington_fan(b, pg, foc=foc)
-            assert want == got and np.isfinite(got).all()
-        assert (RT.trace_astigmatism_coddington_fan(H, fa, wvl, 0.0)
-                == TR.trace_astigmatism_coddington_fan(b, fb, wvl, 0.0, **kw))
+            assert w == got and np.isfinite(got).all()
+        assert want['coddington_astigmatism'] == TR.trace_astigmatism_coddington_fan(b, fb, wvl, 0.0, **kw)
 
-    # OPD of single rays (chief ray present on the field: no re-aiming on either side)
-    for pupil in ([0., 0.6], [0.4, -0.3]):
-        fa.chief_ray = ((None, None, -1.0), None)
+    # OPD of single rays (chief ray present on the field: no re-aiming)
+    for pupil, w in zip(opd_pupils, want['opd']):
         fb.chief_ray = ((None, None, -1.0), None)
-        rw = RT.trace_with_opd(H, list(pupil), fa, wvl, 0.01)
         rg = TR.trace_with_opd(b, list(pupil), fb, wvl, 0.01, **kw)
-        assert rw[1] == rg[1] and rw[2] == rg[2] and rw[3] == rg[3]
-        assert np.array_equal(rw[0][-1][0], rg[0][-1][0])
+        assert w[0] == rg[1] and w[1] == rg[2] and w[2] == rg[3]
+        assert np.array_equal(w[3], rg[0][-1][0])
 
     # DataFrames
-    dw, dg = RT.trace_all_fields(H), TR.trace_all_fields(b, **kw)
-    assert list(dw.index) == list(dg.index) and list(dw.columns) == list(dg.columns)
-    for col in dw.columns:
-        for x, y in zip(dw[col], dg[col]):
-            assert np.array_equal(np.asarray(x), np.asarray(y))
-    assert TR.ray_pkg(pg).index.tolist() == RT.ray_pkg(pw).index.tolist()
+    assert df_values(TR.trace_all_fields(b, **kw)) == want['all_fields']
+    assert TR.ray_pkg(pg).index.tolist() == want['ray_pkg_index']
 
     # printers
     capsys.readouterr()
-    RT.list_ray(pw)
-    RT.list_ray((pw, None), tfrms=[(np.identity(3), np.array([0., 0., float(k)])) for k in range(len(pw.ray))], start=2)
-    RT.list_in_out_dir(list(H.seq_model.path(wvl)), pw.ray)
-    want = capsys.readouterr().out
     TR.list_ray(pg)
     TR.list_ray((pg, None), tfrms=[(np.identity(3), np.array([0., 0., float(k)])) for k in range(len(pg.ray))], start=2)
     TR.list_in_out_dir(list(b.seq_model.path(wvl)), pg.ray)
     got = capsys.readouterr().out
-    assert want == got and len(got.splitlines()) > 2*len(pg.ray)
+    assert want['printed'] == got and len(got.splitlines()) > 2*len(pg.ray)
 
-    P1, V1 = np.array([0., 1., 0.]), np.array([0., -0.1, 1.])/np.linalg.norm([0., -0.1, 1.])
-    P2, V2 = np.array([0., -1., 0.]), np.array([0., 0.1, 1.])/np.linalg.norm([0., 0.1, 1.])
-    assert RT.intersect_2_lines(P1, V1, P2, V2) == TR.intersect_2_lines(P1, V1, P2, V2)
+    assert want['intersect'] == TR.intersect_2_lines(P1, V1, P2, V2)
 
 
-@needs_ref
 @pytest.mark.parametrize('name,use_parax', [('dblgauss', False), ('dblgauss', True), ('triplet', False),
                                             ('relay_fno', False)])
-def test_set_pupil_and_bisection_equal_the_references(name, use_parax, capsys):
+def test_set_pupil_and_bisection_equal_the_references(name, use_parax, capsys, ref):
     """vigcalc.set_pupil (stop size -> pupil specification + vignetting), set_stop_aperture and
     calc_vignetted_ray_by_bisection against rayoptics.raytr.vigcalc on the hybrid model."""
-    import importlib
-    from oracle import ref_model
+    import contextlib
+    import io
     from rayoptics_b200 import vigcalc as V
-    ref_model.modules()
-    RV = importlib.import_module('rayoptics.raytr.vigcalc')
-    a, b = load_model(name), load_model(name)
-    H = ref_model.HybridModel(a)
-    H.update_model = a.update_model
-    kw = dict(tracer=oracle_tracer)
+    starts = ((1, [0., 1.]), (0, [-1., 0.]))
 
-    def keep():
-        for f in a.optical_spec.field_of_view.fields:
-            f.chief_ray = ((None, None, -1.0), None)
-    # bisection search of the upper y pupil edge of the outer field
-    fa, fb = a.optical_spec.field_of_view.fields[-1], b.optical_spec.field_of_view.fields[-1]
-    wvl = a.seq_model.central_wavelength()
-    for xy, start in ((1, [0., 1.]), (0, [-1., 0.])):
+    def reference_side():
+        import importlib
+        from oracle import ref_model
+        ref_model.modules()
+        RV = importlib.import_module('rayoptics.raytr.vigcalc')
+        a = load_model(name)
+        H = ref_model.HybridModel(a)
+        H.update_model = a.update_model
+
+        def keep():
+            for f in a.optical_spec.field_of_view.fields:
+                f.chief_ray = ((None, None, -1.0), None)
+        # bisection search of the upper y pupil edge of the outer field
+        fa = a.optical_spec.field_of_view.fields[-1]
+        wvl = a.seq_model.central_wavelength()
+        bisection = []
+        for xy, start in starts:
+            keep()
+            vw, cw, pw = RV.calc_vignetted_ray_by_bisection(H, xy, np.array(start), fa, wvl)
+            bisection.append((vw, cw, len(pw[0])))
+        # a smaller stop: the pupil specification follows
+        stop = a.seq_model.stop_surface
+        r = 0.9*a.seq_model.ifcs[stop].max_aperture
+        H.seq_model.ifcs[stop].set_max_aperture(r)
+        a.seq_model.ifcs[stop].set_max_aperture(r)
         keep()
-        vw, cw, pw = RV.calc_vignetted_ray_by_bisection(H, xy, np.array(start), fa, wvl)
+        a_update = a.update_model
+
+        def update_and_keep(**k):
+            a_update(**k)
+            keep()
+        H.update_model = update_and_keep
+        text = io.StringIO()
+        with contextlib.redirect_stdout(text):
+            RV.set_pupil(H, use_parax=use_parax)
+        return {'bisection': bisection, 'pupil': a.optical_spec.pupil.value,
+                'axial_limited': text.getvalue().count('Axial bundle limited'),
+                'vig': [(f.vux, f.vlx, f.vuy, f.vly) for f in a.optical_spec.field_of_view.fields]}
+    want = ref(reference_side)
+    capsys.readouterr()
+    b = load_model(name)
+    kw = dict(tracer=oracle_tracer)
+    fb = b.optical_spec.field_of_view.fields[-1]
+    wvl = b.seq_model.central_wavelength()
+    for (xy, start), (vw, cw, n_pw) in zip(starts, want['bisection']):
         vg, cg, pg = V.calc_vignetted_ray_by_bisection(b, xy, np.array(start), fb, wvl, **kw)
-        assert vw == vg and cw == cg and len(pw[0]) == len(pg[0])
+        assert vw == vg and cw == cg and n_pw == len(pg[0])
     # a smaller stop: the pupil specification follows
-    stop = a.seq_model.stop_surface
+    stop = b.seq_model.stop_surface
     r = 0.9*b.seq_model.ifcs[stop].max_aperture
-    H.seq_model.ifcs[stop].set_max_aperture(r)
-    a.seq_model.ifcs[stop].set_max_aperture(r)
     b.seq_model.ifcs[stop].set_max_aperture(r)
     before = b.optical_spec.pupil.value
-    keep()
-    a_update = a.update_model
-
-    def update_and_keep(**k):
-        a_update(**k)
-        keep()
-    H.update_model = update_and_keep
-    RV.set_pupil(H, use_parax=use_parax)
     V.set_pupil(b, use_parax=use_parax, **kw)
-    assert a.optical_spec.pupil.value == b.optical_spec.pupil.value != before
+    assert want['pupil'] == b.optical_spec.pupil.value != before
     # (the reference's image-space f/# comes out negative for the relay: kept, it is its number)
     assert abs(abs(b.optical_spec.pupil.value/before) - (1/0.9 if b.optical_spec.pupil.key[1] == 'f/#' else 0.9)) < 0.02
-    for x, y in zip(a.optical_spec.field_of_view.fields, b.optical_spec.field_of_view.fields):
-        assert (x.vux, x.vlx, x.vuy, x.vly) == (y.vux, y.vlx, y.vuy, y.vly)
-    assert capsys.readouterr().out.count('Axial bundle limited') in (0, 2)
+    assert want['vig'] == [(y.vux, y.vlx, y.vuy, y.vly) for y in b.optical_spec.field_of_view.fields]
+    assert capsys.readouterr().out.count('Axial bundle limited') == want['axial_limited']
 
 
 def oracle_trace_fn(opm):
@@ -817,15 +910,12 @@ def test_aperture_lists_and_stop_aperture():
     assert orig[stop] > 0
 
 
-@needs_ref
 @pytest.mark.parametrize('name,fi', [('dblgauss', 2), ('triplet', 1), ('evenasph', 1)])
-def test_iterate_ray_raw_equals_the_references(name, fi):
+def test_iterate_ray_raw_equals_the_references(name, fi, ref):
     """vigcalc.iterate_ray_raw against rayoptics.raytr.trace.iterate_ray_raw (imported, run on
     the reference's own trace_raw over reference surfaces): same aim point, 1-D (newton) and
     2-D (fsolve) branches."""
-    from oracle import ref_model, ref_harness as rh
     from rayoptics_b200 import vigcalc as V
-    RT, RA = ref_model.modules()
     opm = load_model(name)
     sm, osp = opm.seq_model, opm.optical_spec
     fod = osp.fod
@@ -834,50 +924,67 @@ def test_iterate_ray_raw_equals_the_references(name, fi):
     pt0, d0 = osp.obj_coords(fld)
     one = oracle_trace_fn(opm)
     args = (fod.obj_dist + fod.enp_dist, fod.enp_radius, wvl, True)
-    for target, p0 in ((np.array([0., 0.]), pt0), (np.array([0.05, -0.02]), pt0),
-                       (np.array([0., 0.1]), pt0 + np.array([0.3, 0., 0.]))):
-        want, rr_w = RT.iterate_ray_raw(rh.ref_path(sm, wvl), sm.stop_surface, target, p0, d0, *args)
+    cases = ((np.array([0., 0.]), pt0), (np.array([0.05, -0.02]), pt0),
+             (np.array([0., 0.1]), pt0 + np.array([0.3, 0., 0.])))
+
+    def reference_side():
+        from oracle import ref_model, ref_harness as rh
+        RT, RA = ref_model.modules()
+        out = []
+        for target, p0 in cases:
+            want, rr_w = RT.iterate_ray_raw(rh.ref_path(sm, wvl), sm.stop_surface, target, p0, d0, *args)
+            out.append((want, rr_w.pkg.ray[-1][0]))
+        return out
+    for (target, p0), (want, p_last) in zip(cases, ref(reference_side)):
         got, rr_g = V.iterate_ray_raw(sm.path(wvl), sm.stop_surface, target, p0, d0, *args,
                                       trace_raw_fn=lambda path, p, d, w: one(sm, p, d, w))
         assert np.array_equal(want, got), (name, target)
-        assert rr_g[1] is None and np.array_equal(rr_w.pkg.ray[-1][0], rr_g[0][0][-1][0])
+        assert rr_g[1] is None and np.array_equal(p_last, rr_g[0][0][-1][0])
     got, rr = V.iterate_ray_raw(sm.path(wvl), None, np.array([0.1, 0.2]), pt0, d0, *args)
     assert np.array_equal(got, [0.1, 0.2]) and rr is None
 
 
-@needs_ref
 @pytest.mark.parametrize('name', ['dblgauss', 'triplet', 'rc', 'cellphone'])
-def test_paraxial_vignetting_equals_the_references(name):
+def test_paraxial_vignetting_equals_the_references(name, ref):
     """vigcalc.paraxial_vignetting / apply_paraxial_vignetting against the reference's METHOD TEXT
     (parax/paraxialdesign.py:1023-1050 -- the module needs opticalglass to import) and
     rayoptics.raytr.trace.apply_paraxial_vignetting run on shims of the same paraxial data."""
-    import ast
-    from oracle import ref_model, ref_harness as rh
     from rayoptics_b200 import vigcalc as V
-    RT, RA = ref_model.modules()
-    src = open('/root/reference/src/rayoptics/parax/paraxialdesign.py').read()
-    cls = [n for n in ast.parse(src).body if isinstance(n, ast.ClassDef) and n.name == 'ParaxialModel'][0]
-    fn = [f for f in cls.body if isinstance(f, ast.FunctionDef) and f.name == 'paraxial_vignetting'][0]
-    ns = dict(mc=type('mc', (), {'ht': 0, 'slp': 1}))
-    exec(ast.get_source_segment(src, fn), ns)
-    a, b = load_model(name), load_model(name)
-    for m in (a, b):                                   # tighter apertures so that something vignettes
+    rels = (0.0, 0.5, 1.0)
+
+    def tighter(m):                                    # tighter apertures so that something vignettes
         for ifc in m.seq_model.ifcs[1:-1]:
             ifc.set_max_aperture(0.8*ifc.max_aperture)
-    H = ref_model.HybridModel(a)
-    for ref_ifc, ifc in zip(H.seq_model.ifcs, a.seq_model.ifcs):
-        ref_ifc.set_max_aperture(ifc.max_aperture)
-    fod = a.optical_spec.fod
-    pm = type('PM', (), {})()
-    pm.seq_model, pm.ax, pm.pr = H.seq_model, fod.ax_ray, fod.pr_ray
-    pm.paraxial_vignetting = lambda rel_fov=1: ns['paraxial_vignetting'](pm, rel_fov)
-    for rel in (0.0, 0.5, 1.0):
-        assert pm.paraxial_vignetting(rel) == V.paraxial_vignetting(b, rel)
-    H.parax_model = pm
-    RT.apply_paraxial_vignetting(H)
+        return m
+
+    def reference_side():
+        import ast
+        from oracle import ref_model, ref_harness as rh
+        RT, RA = ref_model.modules()
+        src = open(os.path.join(rh.REF_SRC, 'rayoptics', 'parax', 'paraxialdesign.py')).read()
+        cls = [n for n in ast.parse(src).body if isinstance(n, ast.ClassDef) and n.name == 'ParaxialModel'][0]
+        fn = [f for f in cls.body if isinstance(f, ast.FunctionDef) and f.name == 'paraxial_vignetting'][0]
+        ns = dict(mc=type('mc', (), {'ht': 0, 'slp': 1}))
+        exec(ast.get_source_segment(src, fn), ns)
+        a = tighter(load_model(name))
+        H = ref_model.HybridModel(a)
+        for ref_ifc, ifc in zip(H.seq_model.ifcs, a.seq_model.ifcs):
+            ref_ifc.set_max_aperture(ifc.max_aperture)
+        fod = a.optical_spec.fod
+        pm = type('PM', (), {})()
+        pm.seq_model, pm.ax, pm.pr = H.seq_model, fod.ax_ray, fod.pr_ray
+        pm.paraxial_vignetting = lambda rel_fov=1: ns['paraxial_vignetting'](pm, rel_fov)
+        vig = [pm.paraxial_vignetting(rel) for rel in rels]
+        H.parax_model = pm
+        RT.apply_paraxial_vignetting(H)
+        return vig, [(f.vly, f.vuy) for f in a.optical_spec.field_of_view.fields]
+    want_vig, want_fields = ref(reference_side)
+    b = tighter(load_model(name))
+    for rel, w in zip(rels, want_vig):
+        assert w == V.paraxial_vignetting(b, rel)
     TR.apply_paraxial_vignetting(b)
     got = [(f.vly, f.vuy) for f in b.optical_spec.field_of_view.fields]
-    assert [(f.vly, f.vuy) for f in a.optical_spec.field_of_view.fields] == got
+    assert want_fields == got
     assert any(v != 0 for pair in got for v in pair)
 
 
@@ -918,25 +1025,30 @@ def _real_height_model(name):
     return opm, hts
 
 
-@needs_ref
 @pytest.mark.parametrize('name', ['dblgauss', 'triplet', 'relay_fno', 'cellphone'])
-def test_real_image_height_fields_equal_the_references(name):
+def test_real_image_height_fields_equal_the_references(name, ref):
     """('image', 'real height') fields (Zemax FTYP 3): wideangle.eval_real_image_ht -- the chief ray
     iterated backwards through the stop centre on SequentialModel.reverse_path -- against the
     reference's own eval_real_image_ht (its iterate_ray_raw, its trace_raw on reference surfaces in
     the reversed path); then obj_coords / ray_start_from_osp: the forward chief ray lands on the
     requested image height."""
-    import importlib
-    from oracle import ref_model
     from rayoptics_b200 import wideangle as W
-    ref_model.modules()
-    RW = importlib.import_module('rayoptics.raytr.wideangle')
-    (a, hts), (b, _) = _real_height_model(name), _real_height_model(name)
-    H = ref_model.HybridModel(a)
-    wvl = a.seq_model.central_wavelength()
+
+    def reference_side():
+        import importlib
+        from oracle import ref_model
+        ref_model.modules()
+        RW = importlib.import_module('rayoptics.raytr.wideangle')
+        a, _ = _real_height_model(name)
+        H = ref_model.HybridModel(a)
+        wvl = a.seq_model.central_wavelength()
+        return [RW.eval_real_image_ht(H, fa, wvl) for fa in a.optical_spec.field_of_view.fields]
+    want = ref(reference_side)
+    b, hts = _real_height_model(name)
+    wvl = b.seq_model.central_wavelength()
     b.optical_spec._trace_raw_fn = oracle_trace_raw_fn
-    for fa, fb, h in zip(a.optical_spec.field_of_view.fields, b.optical_spec.field_of_view.fields, hts):
-        (pw, dw), zw = RW.eval_real_image_ht(H, fa, wvl)
+    assert len(want) == len(b.optical_spec.field_of_view.fields)
+    for fb, h, ((pw, dw), zw) in zip(b.optical_spec.field_of_view.fields, hts, want):
         (pg, dg), zg = W.eval_real_image_ht(b, fb, wvl, trace_raw_fn=oracle_trace_raw_fn)
         assert np.array_equal(pw, pg) and np.array_equal(dw, dg) and zw == zg
         # forward: the start ray built from obj_coords (which stores the implied aim point) hits h
@@ -967,14 +1079,13 @@ def test_real_image_height_fields_equal_the_references(name):
                 k += 1
 
 
-@needs_ref
 @pytest.mark.parametrize('fname', ['zemax/tests/US05831776-1.zmx', 'zemax/tests/US08427765-1.ZMX'])
 def test_zemax_real_image_height_files(fname):
     """The two bundled Zemax files with FTYP 3 (fields given as real image heights): the chief ray
     of every field lands on its height and passes the stop centre."""
     import warnings
     from rayoptics_b200 import zmx, seq
-    opm = zmx.open_zmx('/root/reference/src/rayoptics/' + fname, glass_map=seq.SubstituteGlasses())
+    opm = zmx.open_zmx(os.path.join(lens_files(), fname), glass_map=seq.SubstituteGlasses())
     osp, sm = opm.optical_spec, opm.seq_model
     assert tuple(osp.field_of_view.key) == ('image', 'real height')
     osp._trace_raw_fn = oracle_trace_raw_fn
@@ -1022,22 +1133,15 @@ def test_engine_failures_stay_loud_inside_the_searches():
     assert not V.solver_gave_up(_abi.EngineError('Failed to converge'))     # not scipy's class
 
 
-@needs_ref
-def test_real_pupil_search_decisions_equal_the_references(monkeypatch):
+def test_real_pupil_search_decisions_equal_the_references(monkeypatch, ref):
     """Every branch of the wide-angle pupil search (scan direction reversal, first-surface misses,
     single success, beam edges, no crossing) against the reference's find_real_enp: both run on the
     same SYNTHETIC 'ray' -- a scripted stop height h(z) with windows where the trace fails in
     scripted ways -- substituted for enp_z_coordinate in the two modules.  Same z_enp, same
-    sequence of z values evaluated."""
-    import importlib
+    sequence of z values evaluated (stored as their count per scenario and one digest())."""
     import warnings
-    from oracle import ref_model, ref_harness as rh
     from rayoptics_b200 import wideangle as W, raytrace as BR
-    ref_model.modules()
-    RW = importlib.import_module('rayoptics.raytr.wideangle')
-    R = rh.ref()
     opm = load_model('fisheye')
-    H = ref_model.HybridModel(opm)
     stop = opm.seq_model.stop_surface
     wvl = opm.seq_model.central_wavelength()
     fld = opm.optical_spec.field_of_view.fields[3]
@@ -1079,68 +1183,89 @@ def test_real_pupil_search_decisions_equal_the_references(monkeypatch):
             return np.array([0., 0., 0.]), RayResult(RayPkg(ray[:err.surf + 1], 0.0, wvl), err)
         return fn
 
+    scenarios = [scenario() for _ in range(1500)]
+
+    def run(module, model, f, errs, RayPkg, RayResult):
+        """per scenario: z_enp found by module.find_real_enp (or the exception's class name), and
+        the z values it evaluated"""
+        found, logs = [], []
+        for sc in scenarios:
+            log = []
+            monkeypatch.setattr(module, 'enp_z_coordinate', synthetic(sc, errs, RayPkg, RayResult, log))
+            f.aim_info = None
+            with warnings.catch_warnings():
+                warnings.simplefilter('ignore')
+                try:
+                    z = module.find_real_enp(model, stop, f, wvl)[0]
+                except Exception as e:      # noqa: BLE001 - e.g. no successful ray at all: start_z is None
+                    z = type(e).__name__
+            found.append(z)
+            logs.append(log)
+        return found, logs
+
+    def reference_side():
+        import importlib
+        from oracle import ref_model, ref_harness as rh
+        ref_model.modules()
+        RW = importlib.import_module('rayoptics.raytr.wideangle')
+        a = load_model('fisheye')
+        found, logs = run(RW, ref_model.HybridModel(a), a.optical_spec.field_of_view.fields[3],
+                          rh.ref().traceerror, RW.RayPkg, RW.RayResult)
+        return found, [len(log) for log in logs], digest(logs)
+    want, want_counts, want_logs = ref(reference_side)
+    got, logs = run(W, opm, fld, BR, TR.RayPkg, TR.RayResult)
+    assert [len(log) for log in logs] == want_counts and digest(logs) == want_logs
     outcomes = set()
-    for trial in range(1500):
-        sc = scenario()
-        log_r, log_m = [], []
-        monkeypatch.setattr(RW, 'enp_z_coordinate', synthetic(sc, R.traceerror, RW.RayPkg, RW.RayResult, log_r))
-        monkeypatch.setattr(W, 'enp_z_coordinate', synthetic(sc, BR, TR.RayPkg, TR.RayResult, log_m))
-        fld.aim_info = None
-        want = got = None
-        with warnings.catch_warnings():
-            warnings.simplefilter('ignore')
-            try:
-                want = RW.find_real_enp(H, stop, fld, wvl)[0]
-            except Exception as e:      # noqa: BLE001 - e.g. no successful ray at all: start_z is None
-                want = type(e).__name__
-            fld.aim_info = None
-            try:
-                got = W.find_real_enp(opm, stop, fld, wvl)[0]
-            except Exception as e:      # noqa: BLE001
-                got = type(e).__name__
-        assert log_r == log_m, (trial, sc['lo'], sc['hi'], sc['kinds'])
-        assert (want == got) or (isinstance(want, float) and np.isnan(want) and np.isnan(got)), trial
-        outcomes.add('error' if isinstance(want, str) else
-                     'crossing' if abs(sc['h'](want)) < 1e-6 else 'no crossing')
-    assert outcomes == {'error', 'crossing', 'no crossing'}
+    for trial, (sc, w, g) in enumerate(zip(scenarios, want, got)):
+        assert (w == g) or (isinstance(w, float) and np.isnan(w) and np.isnan(g)), trial
+        outcomes.add('error' if isinstance(w, str) else
+                     'crossing' if abs(sc['h'](w)) < 1e-6 else 'no crossing')
+    assert len(got) == len(want) == 1500 and outcomes == {'error', 'crossing', 'no crossing'}
 
 
-@needs_ref
 @pytest.mark.parametrize('name', ['dblgauss', 'relay_na', 'fisheye'])
-def test_aim_point_and_aim_direction_pupils(name):
+def test_aim_point_and_aim_direction_pupils(name, ref):
     """trace_base / trace_safe with pupil_type 'aim pt' and 'aim dir' (trace.py:253-310,
     opticalspec.py:332-336,369-371): the reference's trace_base on the hybrid model against the
-    bundle path here, whole rays."""
-    from oracle import ref_model
-    RT, RA = ref_model.modules()
-    a, b = load_model(name), load_model(name)
-    H = ref_model.HybridModel(a)
-    wvl = a.seq_model.central_wavelength()
-    fod = a.optical_spec.fod
-    fa, fb = a.optical_spec.field_of_view.fields[1], b.optical_spec.field_of_view.fields[1]
-    angular = a.optical_spec.pupil.key[1] != 'epd'
+    bundle path here, whole rays (the segments' p, d, dst as digest())."""
+    b = load_model(name)
+    wvl = b.seq_model.central_wavelength()
+    fod = b.optical_spec.fod
+    fb = b.optical_spec.field_of_view.fields[1]
+    angular = b.optical_spec.pupil.key[1] != 'epd'
     if angular:
         ptype, pupils = 'aim dir', [np.array([0.0, 0.02]), np.array([0.01, -0.015]), np.array([-0.02, 0.0])]
     else:
         r = fod.enp_radius
         ptype, pupils = 'aim pt', [np.array([0.0, 0.3*r]), np.array([0.2*r, -0.4*r]), np.array([-0.5*r, 0.1*r])]
+
+    def summary(pkg):
+        return len(pkg[0]), pkg[1], digest([tuple(seg)[:3] for seg in pkg[0]])
+
+    def reference_side():
+        from oracle import ref_model
+        RT, RA = ref_model.modules()
+        a = load_model(name)
+        H = ref_model.HybridModel(a)
+        fa = a.optical_spec.field_of_view.fields[1]
+        out = []
+        for pupil in pupils:
+            for check in (False, True):
+                try:
+                    out.append(summary(RT.trace_base(H, pupil.copy(), fa, wvl, pupil_type=ptype,
+                                                     check_apertures=check)))
+                except Exception as e:      # noqa: BLE001 - a reference TraceError
+                    out.append(type(e).__name__)
+        return out
+    want = iter(ref(reference_side))
     for pupil in pupils:
         for check in (False, True):
             try:
-                want = RT.trace_base(H, pupil.copy(), fa, wvl, pupil_type=ptype, check_apertures=check)
-            except Exception as e:      # noqa: BLE001 - a reference TraceError
-                want = type(e).__name__
-            try:
-                got = TR.trace_base(b, pupil.copy(), fb, wvl, pupil_type=ptype, check_apertures=check,
-                                    bundle_tracer=oracle_bundle_tracer)
+                got = summary(TR.trace_base(b, pupil.copy(), fb, wvl, pupil_type=ptype, check_apertures=check,
+                                            bundle_tracer=oracle_bundle_tracer))
             except Exception as e:      # noqa: BLE001
                 got = type(e).__name__
-            if isinstance(want, str):
-                assert got == want
-                continue
-            assert len(want[0]) == len(got[0]) and want[1] == got[1]
-            for sw, sg in zip(want[0], got[0]):
-                assert np.array_equal(sw[0], sg[0]) and np.array_equal(sw[1], sg[1]) and sw[2] == sg[2]
+            assert got == next(want)
     res = TR.trace_pupil_rays(b, pupils, fb, wvl, None, 'full', pupil_type=ptype,
                               bundle_tracer=oracle_bundle_tracer)
     assert len(res) == 3 and all(r.pkg is not None for r in res)
@@ -1198,30 +1323,32 @@ def test_post_import_update_sets_aims_and_apertures():
     assert own.update_optical_properties(oracle_bundle_fn(own)) == 0
     assert [i.max_aperture for i in own.seq_model.ifcs] == before
     # Zemax: DIAM kind 0 (automatic semi-diameters) leaves the automatic apertures on
-    root = '/root/reference/src/rayoptics/zemax/tests'
-    if os.path.isdir(root):
-        z = zmx.open_zmx(f'{root}/US05831776-1.zmx', glass_map=seq.SubstituteGlasses())
-        assert z.seq_model.do_apertures in (True, False) and z.seq_model.ifcs[1].max_aperture != 1.0
+    z = zmx.open_zmx(os.path.join(lens_files(), 'zemax', 'tests', 'US05831776-1.zmx'),
+                     glass_map=seq.SubstituteGlasses())
+    assert z.seq_model.do_apertures in (True, False) and z.seq_model.ifcs[1].max_aperture != 1.0
 
 
-@needs_ref
-def test_set_max_aperture_resizes_clear_apertures_like_the_reference():
+def test_set_max_aperture_resizes_clear_apertures_like_the_reference(ref):
     """Surface.set_max_aperture (elem/surface.py:174-179): clear apertures follow, obscurations do not"""
-    from oracle import ref_harness as rh
     from rayoptics_b200 import model as M
-    S = rh.ref().surface
+
+    def reference_side():
+        from oracle import ref_harness as rh
+        S = rh.ref().surface
+        s = S.Surface()
+        s.clear_apertures = [S.Circular(radius=3.0), S.Rectangular(x_half_width=2.0, y_half_width=1.0, x_offset=0.5),
+                             S.Circular(radius=0.4, is_obscuration=True)]
+        s.set_max_aperture(5.25)
+        return (s.max_aperture, (s.clear_apertures[0].radius, s.clear_apertures[2].radius),
+                (s.clear_apertures[1].x_half_width, s.clear_apertures[1].y_half_width))
+    want_max, want_radii, want_half_widths = ref(reference_side)
     own = M.Surface(clear_apertures=[M.Circular(radius=3.0), M.Rectangular(2.0, 1.0, x_offset=0.5),
                                       M.Circular(radius=0.4, is_obscuration=True)])
-    ref = S.Surface()
-    ref.clear_apertures = [S.Circular(radius=3.0), S.Rectangular(x_half_width=2.0, y_half_width=1.0, x_offset=0.5),
-                           S.Circular(radius=0.4, is_obscuration=True)]
     own.set_max_aperture(5.25)
-    ref.set_max_aperture(5.25)
-    assert own.max_aperture == ref.max_aperture == 5.25
-    assert (own.clear_apertures[0].radius, own.clear_apertures[2].radius) == \
-           (ref.clear_apertures[0].radius, ref.clear_apertures[2].radius) == (5.25, 0.4)
+    assert own.max_aperture == want_max == 5.25
+    assert (own.clear_apertures[0].radius, own.clear_apertures[2].radius) == want_radii == (5.25, 0.4)
     assert (own.clear_apertures[1].x_half_width, own.clear_apertures[1].y_half_width) == \
-           (ref.clear_apertures[1].x_half_width, ref.clear_apertures[1].y_half_width) == (5.25, 5.25)
+           want_half_widths == (5.25, 5.25)
 
 
 def oracle_tile_fn(opm):
