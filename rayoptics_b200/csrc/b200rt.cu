@@ -12,7 +12,8 @@
  *
  * The surface table (n_ifc x rt_surface_desc + n_wvl x n_ifc indices) is staged
  * into shared memory once per CTA; CTAs are persistent (grid = SMs x resident
- * CTAs) and walk rays / chunks with a grid stride.
+ * CTAs): the bundle kernels walk rays with a grid stride, the warps of the grid
+ * kernels draw 32-ray work items from a per-launch counter.
  */
 #include <cuda_runtime.h>
 #include <math_constants.h>
@@ -23,6 +24,7 @@
 #include <cstring>
 #include <new>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "rt_device.cuh"
@@ -31,18 +33,12 @@
 
 using namespace b200rt;
 
-#ifndef RT_BLOCK
 #define RT_BLOCK 256          /* threads per CTA = rays per chunk */
-#endif
-#ifndef RT_LEAN_MIN_CTAS
 #define RT_LEAN_MIN_CTAS 3   /* resident CTAs per SM the lean kernels are register-limited for */
-#endif
 #define RT_MAX_STAGE_BYTES (200*1024)
 
 /* ------------------------------------------------------------------ errors */
 static thread_local std::string g_err;
-static thread_local int g_last_grid = 0;      /* CTAs of the grid kernel this thread launched last */
-static thread_local int64_t g_item_off = 0;   /* doubles from scratch to the per-item sums (set by rt_trace_grid) */
 static std::atomic<int64_t> g_launches{0};
 
 static int fail(int code, const char *fmt, const char *a = "", const char *b = "")
@@ -89,7 +85,6 @@ struct rt_table {
     bool lean_poly;          /* lean, with polynomial / toroid profiles (out-of-line Newton) */
     bool wave_ok;            /* interface n_ifc-2 carries no decenter: OPD epilogue applicable */
     size_t lean_bytes;       /* shared memory of the lean plan */
-    bool dynamic;            /* grid kernels draw 32-ray work items from a counter (default) */
     unsigned long long *d_counters;     /* ring of RT_COUNTERS work counters */
     std::atomic<unsigned> next_counter;
 };
@@ -181,16 +176,17 @@ k_trace_bundle(const rt_surface_desc *__restrict__ g_surfs, const double *__rest
 }
 
 /* ---- per-(field, wvl) spot sums.
- * Every thread keeps 15 running values in shared memory (acc[k*RT_BLOCK + tid],
- * conflict-free); when the CTA moves on to another tile (or finishes) each warp
- * shuffle-reduces its lanes and lane 0 writes one 16-double record (15 values +
- * a valid flag) to its slot of the tile.  Slots of a tile: RT_WARPS x SL,
- * SL = min(chunks_per_tile, RT_MAX_GRID); slot = local chunk when
- * chunks_per_tile <= gridDim.x (then a CTA never meets a tile twice), else
- * blockIdx.x (a CTA's chunks of one tile are consecutive => one record).  The
- * scratch buffer is zeroed before the launch, k_reduce_summary adds up the valid
- * records of a tile in slot order: bit-reproducible for a given launch shape,
- * and no CTA barrier / per-chunk shuffle traffic in the trace kernel. */
+ * Records of 16 doubles (15 values + a valid flag); slots of a tile: RT_WARPS x SL,
+ * SL = min(chunks_per_tile, RT_MAX_GRID).  When chunks_per_tile <= gridDim.x
+ * (chunk slots) a warp writes the record of its 32 rays of a chunk straight from
+ * registers, slot = local chunk.  Otherwise every thread keeps the counts and
+ * min / max in shared memory (acc[k*RT_BLOCK + tid], conflict-free); when the warp
+ * moves on to another tile (or finishes) it shuffle-reduces its lanes into its
+ * record of slot blockIdx.x (a warp draws its items in ascending order, so it meets
+ * a tile in one run => one record), and the floating-point sums of each work item
+ * are stored on their own.  The scratch buffer is zeroed before the launch,
+ * k_reduce_summary adds up the valid records of a tile in slot order and the item
+ * sums in item order: bit-reproducible, and no CTA barrier in the trace kernel. */
 #define RT_WARPS (RT_BLOCK/32)
 #define RT_MAX_GRID 2048
 #define RT_ACC 15
@@ -204,23 +200,9 @@ __device__ __forceinline__ void acc_init(double *acc)
             (k == 10 || k == 12) ? CUDART_INF : ((k == 11 || k == 13) ? -CUDART_INF : 0.0);
 }
 
-__device__ __forceinline__ void acc_add(double *acc, int status, double ax, double ay, double op)
-{
-    double *a = acc + threadIdx.x;
-    const int ck = status == RT_RAY_OK ? 0 : (status <= RT_RAY_BLOCKED ? status : 4);
-    a[ck*RT_BLOCK] += 1.0;
-    if (status == RT_RAY_OK) {
-        a[5*RT_BLOCK] += ax; a[6*RT_BLOCK] += ay;
-        a[7*RT_BLOCK] += ax*ax; a[8*RT_BLOCK] += ay*ay; a[9*RT_BLOCK] += ax*ay;
-        a[10*RT_BLOCK] = fmin(a[10*RT_BLOCK], ax); a[11*RT_BLOCK] = fmax(a[11*RT_BLOCK], ax);
-        a[12*RT_BLOCK] = fmin(a[12*RT_BLOCK], ay); a[13*RT_BLOCK] = fmax(a[13*RT_BLOCK], ay);
-        a[14*RT_BLOCK] += op;
-    }
-}
-
-/* dynamic scheduling: only the order-independent columns (counts, min / max) go through the
- * per-thread accumulators; the floating-point sums are reduced per work item (item_sums) */
-__device__ __forceinline__ void acc_add_exact(double *acc, int status, double ax, double ay)
+/* only the order-independent columns (counts, min / max) go through the per-thread
+ * accumulators; the floating-point sums are reduced per work item (item_sums_store) */
+__device__ __forceinline__ void acc_add(double *acc, int status, double ax, double ay)
 {
     double *a = acc + threadIdx.x;
     const int ck = status == RT_RAY_OK ? 0 : (status <= RT_RAY_BLOCKED ? status : 4);
@@ -328,27 +310,16 @@ __device__ __forceinline__ void grid_chunk_loop(const GridDev &G, int64_t chunk_
     int64_t cur_tile = -1;
     if (SUMMARY && !chunk_slots) acc_init(acc);
     const unsigned long long n_items = (unsigned long long)(chunk_end - chunk_begin)*RT_WARPS;
-    int64_t c = chunk_begin + blockIdx.x;
     for (;;) {
-        int slice;                       /* which 32 rays of the chunk this warp takes */
+        /* one work item = 32 consecutive rays: every warp draws its next item from a global
+         * counter, so no warp idles while rays are left (the cost of a chunk varies several-fold
+         * between the pupil centre and its clipped edge) */
         unsigned long long item = 0;
-        if (work_counter) {
-            /* dynamic scheduling, one work item = 32 consecutive rays: every warp draws its next
-             * item from a global counter, so no warp idles while rays are left (the cost of a
-             * chunk varies several-fold between the pupil centre and its clipped edge) */
-            unsigned long long u = 0;
-            if ((threadIdx.x & 31) == 0) u = atomicAdd(work_counter, 1ull);
-            u = __shfl_sync(0xffffffffu, u, 0);
-            if (u >= n_items) break;
-            c = chunk_begin + (int64_t)(u/RT_WARPS);
-            slice = (int)(u % RT_WARPS);
-            item = u;
-        } else {
-            if (c >= chunk_end) break;
-            /* static round robin; the slice a warp takes is a hash of the chunk id, so that no
-             * warp is stuck with the pupil-edge (cheap) or the centre (expensive) end of every chunk */
-            slice = (int)(((threadIdx.x >> 5) + ((unsigned)c*0x9E3779B1u >> 27)) % RT_WARPS);
-        }
+        if ((threadIdx.x & 31) == 0) item = atomicAdd(work_counter, 1ull);
+        item = __shfl_sync(0xffffffffu, item, 0);
+        if (item >= n_items) break;
+        const int64_t c = chunk_begin + (int64_t)(item/RT_WARPS);
+        const int slice = (int)(item % RT_WARPS);     /* which 32 rays of the chunk this warp takes */
         const int64_t tile = c/G.chunks_per_tile;
         const int64_t lc = c - tile*G.chunks_per_tile;
         const int64_t loc = lc*RT_BLOCK + slice*32 + (threadIdx.x & 31);
@@ -386,19 +357,15 @@ __device__ __forceinline__ void grid_chunk_loop(const GridDev &G, int64_t chunk_
                     }
                     out.abr_x[k] = sx; out.abr_y[k] = sy;
                 }
-                if (SUMMARY && !chunk_slots) {
-                    if (work_counter) acc_add_exact(acc, status, ax, ay);
-                    else acc_add(acc, status, ax, ay, op);
-                }
+                if (SUMMARY && !chunk_slots) acc_add(acc, status, ax, ay);
             }
         }
-        /* dynamic schedule: which warp adds which rays varies from run to run, so the sums of every
-         * work item are stored on their own and k_reduce_summary adds them in item order --
-         * the summary stays bit-reproducible */
-        if (SUMMARY && !chunk_slots && work_counter)
+        /* which warp adds which rays varies from run to run, so the sums of every work item are
+         * stored on their own and k_reduce_summary adds them in item order -- the summary stays
+         * bit-reproducible */
+        if (SUMMARY && !chunk_slots)
             item_sums_store(have && status == RT_RAY_OK, ax, ay, op, item_sums + item*RT_ITEM_SUMS);
         if (SUMMARY && chunk_slots) warp_record_from_regs(have, status, ax, ay, op, scratch, tile, lc, sl, slice);
-        if (!work_counter) c += gridDim.x;
     }
     if (SUMMARY && !chunk_slots && cur_tile >= 0) acc_flush(acc, scratch, cur_tile, blockIdx.x, sl);
 }
@@ -706,26 +673,33 @@ static int64_t scratch_head_doubles(const rt_grid *g)
     return (scratch_records(g) + g->n_tiles*RT_RED_SPLIT)*RT_SUMMARY_DOUBLES + g->n_tiles;
 }
 
-template <typename K>
-static int persistent_grid(K kernel, size_t smem, int sm_count, int64_t work_items, int *grid)
-{
-    int per_sm = 0;
-    CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, RT_BLOCK, smem));
-    if (per_sm < 1) per_sm = 1;
-    int64_t g = (int64_t)sm_count*per_sm;
-    if (g > work_items) g = work_items;
-    if (g > RT_MAX_GRID) g = RT_MAX_GRID;
-    if (g < 1) g = 1;
-    *grid = (int)g;
-    return RT_OK;
-}
-
-template <typename K>
-static int prep_kernel(K kernel, size_t smem)
+/* Launch a persistent kernel of RT_BLOCK-thread CTAs: as many CTAs as are resident at once
+ * (occupancy x SMs), but no more than work items or RT_MAX_GRID.  Returns the number of CTAs,
+ * or a negative rt_error code. */
+template <typename K, typename... A>
+static int launch(K kernel, size_t smem, int sm_count, int64_t work_items, cudaStream_t stream,
+                  const A &...args)
 {
     if (smem > 48*1024)
         CUDA_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    return RT_OK;
+    int per_sm = 0;
+    CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, RT_BLOCK, smem));
+    if (per_sm < 1) per_sm = 1;
+    int64_t grid = (int64_t)sm_count*per_sm;
+    if (grid > work_items) grid = work_items;
+    if (grid > RT_MAX_GRID) grid = RT_MAX_GRID;
+    if (grid < 1) grid = 1;
+    kernel<<<(unsigned)grid, RT_BLOCK, smem, stream>>>(args...);
+    g_launches++;
+    CUDA_TRY(cudaGetLastError());
+    return (int)grid;
+}
+
+/* f(std::true_type) or f(std::false_type): a runtime flag as a kernel template argument */
+template <typename F>
+static int with_bool(bool b, F f)
+{
+    return b ? f(std::true_type{}) : f(std::false_type{});
 }
 
 static int check_opts(const rt_table *t, const rt_opts *o)
@@ -735,120 +709,13 @@ static int check_opts(const rt_table *t, const rt_opts *o)
     return RT_OK;
 }
 
-template <bool FULL, bool STAGE>
-static int launch_bundle(const rt_table *t, int64_t n_rays, const double *px, const double *py,
-                         const double *pz, const double *dx, const double *dy, const double *dz,
-                         const int32_t *wvl_idx, const rt_opts *o, const rt_out *out,
-                         cudaStream_t stream)
-{
-    auto kern = k_trace_bundle<FULL, STAGE>;
-    const size_t smem = STAGE ? t->stage_bytes : 0;
-    int rc = prep_kernel(kern, smem);
-    if (rc) return rc;
-    int grid;
-    rc = persistent_grid(kern, smem, t->sm_count, (n_rays + RT_BLOCK - 1)/RT_BLOCK, &grid);
-    if (rc) return rc;
-    kern<<<grid, RT_BLOCK, smem, stream>>>(t->d_surfs, t->d_n, t->n_ifc, t->n_wvl, n_rays,
-                                           px, py, pz, dx, dy, dz, wvl_idx, *o, *out, t->d_wvl);
-    g_launches++;
-    CUDA_TRY(cudaGetLastError());
-    return RT_OK;
-}
-
-/* work counter of one launch (NULL: static schedule): a slot of the table's ring, zeroed on the stream */
+/* work counter of one launch: a slot of the table's ring, zeroed on the stream */
 static int launch_counter(const rt_table *t, cudaStream_t stream, unsigned long long **out)
 {
-    *out = nullptr;
-    if (!t->dynamic) return RT_OK;
     rt_table *tt = const_cast<rt_table *>(t);
-    unsigned long long *c = t->d_counters + (tt->next_counter++ % RT_COUNTERS);
-    CUDA_TRY(cudaMemsetAsync(c, 0, sizeof(unsigned long long), stream));
-    *out = c;
+    *out = t->d_counters + (tt->next_counter++ % RT_COUNTERS);
+    CUDA_TRY(cudaMemsetAsync(*out, 0, sizeof(unsigned long long), stream));
     return RT_OK;
-}
-
-template <bool FULL, bool SUMMARY, bool STAGE, bool WAVE = false>
-static int launch_grid(const rt_table *t, const rt_grid *g, const GridDev &G, int64_t cb, int64_t ce,
-                       const rt_opts *o, const rt_out *out, double *scratch, cudaStream_t stream)
-{
-    auto kern = k_trace_grid<FULL, SUMMARY, STAGE, WAVE>;
-    const size_t smem = (STAGE ? t->stage_bytes : 0) + (SUMMARY ? RT_ACC_BYTES : 0);
-    int rc = prep_kernel(kern, smem);
-    if (rc) return rc;
-    int grid;
-    rc = persistent_grid(kern, smem, t->sm_count, ce - cb, &grid);
-    if (rc) return rc;
-    unsigned long long *wc;
-    rc = launch_counter(t, stream, &wc);
-    if (rc) return rc;
-    g_last_grid = grid;
-    kern<<<grid, RT_BLOCK, smem, stream>>>(t->d_surfs, t->d_n, t->n_ifc, t->n_wvl, G, cb, ce, *o, *out,
-                                           scratch, t->d_wvl, g->pupil_kind, wc,
-                                           (wc && SUMMARY) ? scratch + g_item_off : nullptr);
-    g_launches++;
-    CUDA_TRY(cudaGetLastError());
-    return RT_OK;
-}
-
-template <int OUT, bool POLY>
-static int launch_bundle_lean_(const rt_table *t, int64_t n_rays, const double *px, const double *py,
-                              const double *pz, const double *dx, const double *dy, const double *dz,
-                              const int32_t *wvl_idx, const rt_opts *o, const rt_out *out,
-                              cudaStream_t stream)
-{
-    auto kern = k_trace_bundle_lean<OUT, POLY>;   /* (lean kernels: no phase elements, no wavelengths) */
-    const size_t smem = t->lean_bytes;
-    int rc = prep_kernel(kern, smem);
-    if (rc) return rc;
-    int grid;
-    rc = persistent_grid(kern, smem, t->sm_count, (n_rays + RT_BLOCK - 1)/RT_BLOCK, &grid);
-    if (rc) return rc;
-    kern<<<grid, RT_BLOCK, smem, stream>>>(t->d_surfs, t->d_n, t->n_ifc, t->n_wvl, n_rays,
-                                           px, py, pz, dx, dy, dz, wvl_idx, *o, *out);
-    g_launches++;
-    CUDA_TRY(cudaGetLastError());
-    return RT_OK;
-}
-
-template <int OUT, bool SUMMARY, bool WAVE, bool POLY>
-static int launch_grid_lean_(const rt_table *t, const GridDev &G, int64_t cb, int64_t ce,
-                            const rt_opts *o, const rt_out *out, double *scratch, cudaStream_t stream)
-{
-    auto kern = k_trace_grid_lean<OUT, SUMMARY, WAVE, POLY>;
-    const size_t smem = t->lean_bytes + (SUMMARY ? RT_ACC_BYTES : 0);
-    int rc = prep_kernel(kern, smem);
-    if (rc) return rc;
-    int grid;
-    rc = persistent_grid(kern, smem, t->sm_count, ce - cb, &grid);
-    if (rc) return rc;
-    unsigned long long *wc;
-    rc = launch_counter(t, stream, &wc);
-    if (rc) return rc;
-    g_last_grid = grid;
-    kern<<<grid, RT_BLOCK, smem, stream>>>(t->d_surfs, t->d_n, t->n_ifc, t->n_wvl, G, cb, ce, *o, *out,
-                                           scratch, wc, (wc && SUMMARY) ? scratch + g_item_off : nullptr);
-    g_launches++;
-    CUDA_TRY(cudaGetLastError());
-    return RT_OK;
-}
-
-template <int OUT>
-static int launch_bundle_lean(const rt_table *t, int64_t n_rays, const double *px, const double *py,
-                              const double *pz, const double *dx, const double *dy, const double *dz,
-                              const int32_t *wvl_idx, const rt_opts *o, const rt_out *out,
-                              cudaStream_t stream)
-{
-    return t->lean_poly
-        ? launch_bundle_lean_<OUT, true>(t, n_rays, px, py, pz, dx, dy, dz, wvl_idx, o, out, stream)
-        : launch_bundle_lean_<OUT, false>(t, n_rays, px, py, pz, dx, dy, dz, wvl_idx, o, out, stream);
-}
-
-template <int OUT, bool SUMMARY, bool WAVE = false>
-static int launch_grid_lean(const rt_table *t, const GridDev &G, int64_t cb, int64_t ce,
-                            const rt_opts *o, const rt_out *out, double *scratch, cudaStream_t stream)
-{
-    return t->lean_poly ? launch_grid_lean_<OUT, SUMMARY, WAVE, true>(t, G, cb, ce, o, out, scratch, stream)
-                        : launch_grid_lean_<OUT, SUMMARY, WAVE, false>(t, G, cb, ce, o, out, scratch, stream);
 }
 
 /* 0: p,d only; 1: + normal/dst; 2: whole ray */
@@ -857,6 +724,17 @@ static int out_kind(const rt_out *out)
     if (out->full) return 2;
     if (out->nx || out->ny || out->nz || out->dst) return 1;
     return 0;
+}
+
+/* f(std::integral_constant<int, out_kind(out)>): the lean kernels' output kind as a template argument */
+template <typename F>
+static int with_out_kind(const rt_out *out, F f)
+{
+    switch (out_kind(out)) {
+    case 0: return f(std::integral_constant<int, 0>{});
+    case 1: return f(std::integral_constant<int, 1>{});
+    default: return f(std::integral_constant<int, 2>{});
+    }
 }
 
 static GridDev grid_dev(const rt_grid *g)
@@ -922,9 +800,6 @@ int rt_table_create(const rt_surface_desc *surfs, int32_t n_ifc, const double *n
         if (t->lean_bytes > RT_MAX_STAGE_BYTES - RT_ACC_BYTES) t->lean = false;
     }
     if (getenv("B200RT_NO_LEAN")) t->lean = false;
-    /* grid kernels: warps draw 32-ray work items from a counter (B200RT_STATIC=1: fixed round robin
-     * of chunks over CTAs, the round-1 schedule, kept for comparison -- profiles/r02*) */
-    t->dynamic = getenv("B200RT_STATIC") == nullptr;
     t->d_counters = nullptr; t->next_counter = 0;
     {
         const rt_surface_desc &k = surfs[n_ifc >= 2 ? n_ifc - 2 : 0];
@@ -995,19 +870,26 @@ int rt_trace_bundle(const rt_table *t, int64_t n_rays, const double *px, const d
         return fail(RT_ERR_INVALID, "rt_trace_bundle: full_stride < n_rays");
     DeviceGuard guard(t->device);
     cudaStream_t s = (cudaStream_t)stream;
-    if (t->lean) {
-        switch (out_kind(out)) {
-        case 0: return launch_bundle_lean<0>(t, n_rays, px, py, pz, dx, dy, dz, wvl_idx, o, out, s);
-        case 1: return launch_bundle_lean<1>(t, n_rays, px, py, pz, dx, dy, dz, wvl_idx, o, out, s);
-        default: return launch_bundle_lean<2>(t, n_rays, px, py, pz, dx, dy, dz, wvl_idx, o, out, s);
-        }
+    const int64_t chunks = (n_rays + RT_BLOCK - 1)/RT_BLOCK;
+    int grid;
+    if (t->lean) {                  /* (lean kernels: no phase elements, no wavelengths) */
+        grid = with_out_kind(out, [&](auto kind) {
+            return with_bool(t->lean_poly, [&](auto poly) {
+                return launch(k_trace_bundle_lean<kind, poly>, t->lean_bytes, t->sm_count, chunks, s,
+                              t->d_surfs, t->d_n, t->n_ifc, t->n_wvl, n_rays, px, py, pz, dx, dy, dz,
+                              wvl_idx, *o, *out);
+            });
+        });
+    } else {
+        grid = with_bool(out->full != nullptr, [&](auto full) {
+            return with_bool(t->stage, [&](auto stage) {
+                return launch(k_trace_bundle<full, stage>, stage ? t->stage_bytes : 0, t->sm_count, chunks, s,
+                              t->d_surfs, t->d_n, t->n_ifc, t->n_wvl, n_rays, px, py, pz, dx, dy, dz,
+                              wvl_idx, *o, *out, t->d_wvl);
+            });
+        });
     }
-    if (out->full) {
-        return t->stage ? launch_bundle<true, true>(t, n_rays, px, py, pz, dx, dy, dz, wvl_idx, o, out, s)
-                        : launch_bundle<true, false>(t, n_rays, px, py, pz, dx, dy, dz, wvl_idx, o, out, s);
-    }
-    return t->stage ? launch_bundle<false, true>(t, n_rays, px, py, pz, dx, dy, dz, wvl_idx, o, out, s)
-                    : launch_bundle<false, false>(t, n_rays, px, py, pz, dx, dy, dz, wvl_idx, o, out, s);
+    return grid < 0 ? grid : RT_OK;
 }
 
 int rt_grid_destroy(rt_grid *g)
@@ -1162,11 +1044,9 @@ int rt_trace_grid(const rt_table *t, const rt_grid *g, int64_t chunk_begin, int6
     if (chunk_begin == chunk_end) return RT_OK;
     const GridDev G = grid_dev(g);
     double *scr = (double *)scratch;
-    g_item_off = scratch_head_doubles(g);
     if (summary)
-        CUDA_TRY(cudaMemsetAsync(scr, 0, (size_t)(t->dynamic ? rt_grid_scratch_bytes(g, chunk_begin, chunk_end)
-                                                              : scratch_head_doubles(g)*(int64_t)sizeof(double)), s));
-    const bool full = out->full != nullptr, summ = summary != nullptr, st = t->stage;
+        CUDA_TRY(cudaMemsetAsync(scr, 0, (size_t)rt_grid_scratch_bytes(g, chunk_begin, chunk_end), s));
+    const bool summ = summary != nullptr;
     const bool wave = out->opd != nullptr;
     /* angular pupil specifications are generated by the general kernels only (rt_grid.cuh) */
     const bool lean = t->lean && g->pupil_kind == RT_PUPIL_EPD;
@@ -1175,48 +1055,49 @@ int rt_trace_grid(const rt_table *t, const rt_grid *g, int64_t chunk_begin, int6
         if (out_kind(out) != 0) return fail(RT_ERR_UNSUPPORTED, "rt_trace_grid: opd cannot be combined with normals / whole rays");
         if (!t->wave_ok)
             return fail(RT_ERR_UNSUPPORTED, "rt_trace_grid: opd needs >= 3 interfaces and no decenter on the last one before the image");
-        if (lean) {
-            rc = summ ? launch_grid_lean<0, true, true>(t, G, chunk_begin, chunk_end, o, out, scr, s)
-                      : launch_grid_lean<0, false, true>(t, G, chunk_begin, chunk_end, o, out, scr, s);
-        } else if (st) {
-            rc = summ ? launch_grid<false, true, true, true>(t, g, G, chunk_begin, chunk_end, o, out, scr, s)
-                      : launch_grid<false, false, true, true>(t, g, G, chunk_begin, chunk_end, o, out, scr, s);
-        } else {
-            rc = summ ? launch_grid<false, true, false, true>(t, g, G, chunk_begin, chunk_end, o, out, scr, s)
-                      : launch_grid<false, false, false, true>(t, g, G, chunk_begin, chunk_end, o, out, scr, s);
-        }
-    } else if (lean) {
-        const int kind = out_kind(out);
-#define RT_LEAN_CASE(K, S)                                                                   \
-        if (kind == K && summ == S)                                                          \
-            rc = launch_grid_lean<K, S>(t, G, chunk_begin, chunk_end, o, out, scr, s);
-        RT_LEAN_CASE(0, false) RT_LEAN_CASE(0, true) RT_LEAN_CASE(1, false)
-        RT_LEAN_CASE(1, true) RT_LEAN_CASE(2, false) RT_LEAN_CASE(2, true)
-#undef RT_LEAN_CASE
-    } else {
-#define RT_GRID_CASE(F, S, T)                                                               \
-    if (full == F && summ == S && st == T)                                                  \
-        rc = launch_grid<F, S, T>(t, g, G, chunk_begin, chunk_end, o, out, scr, s);
-    RT_GRID_CASE(false, false, true)
-    RT_GRID_CASE(false, true, true)
-    RT_GRID_CASE(true, false, true)
-    RT_GRID_CASE(true, true, true)
-    RT_GRID_CASE(false, false, false)
-    RT_GRID_CASE(false, true, false)
-    RT_GRID_CASE(true, false, false)
-    RT_GRID_CASE(true, true, false)
-#undef RT_GRID_CASE
     }
+    unsigned long long *wc;
+    rc = launch_counter(t, s, &wc);
     if (rc) return rc;
+    double *item_sums = summ ? scr + scratch_head_doubles(g) : nullptr;
+    const int64_t cb = chunk_begin, ce = chunk_end;
+    auto launch_lean = [&](auto kind, auto wave_c) {
+        return with_bool(summ, [&](auto summ_c) {
+            return with_bool(t->lean_poly, [&](auto poly) {
+                return launch(k_trace_grid_lean<kind, summ_c, wave_c, poly>,
+                              t->lean_bytes + (summ_c ? RT_ACC_BYTES : 0), t->sm_count, ce - cb, s,
+                              t->d_surfs, t->d_n, t->n_ifc, t->n_wvl, G, cb, ce, *o, *out, scr, wc, item_sums);
+            });
+        });
+    };
+    auto launch_general = [&](auto full, auto wave_c) {
+        return with_bool(summ, [&](auto summ_c) {
+            return with_bool(t->stage, [&](auto stage) {
+                return launch(k_trace_grid<full, summ_c, stage, wave_c>,
+                              (stage ? t->stage_bytes : 0) + (summ_c ? RT_ACC_BYTES : 0), t->sm_count, ce - cb, s,
+                              t->d_surfs, t->d_n, t->n_ifc, t->n_wvl, G, cb, ce, *o, *out, scr, t->d_wvl,
+                              g->pupil_kind, wc, item_sums);
+            });
+        });
+    };
+    int grid;
+    if (wave)
+        grid = lean ? launch_lean(std::integral_constant<int, 0>{}, std::true_type{})
+                    : launch_general(std::false_type{}, std::true_type{});
+    else if (lean)
+        grid = with_out_kind(out, [&](auto kind) { return launch_lean(kind, std::false_type{}); });
+    else
+        grid = with_bool(out->full != nullptr, [&](auto full) { return launch_general(full, std::false_type{}); });
+    if (grid < 0) return grid;
     if (summ) {
         const int64_t recs = scratch_records(g);
         double *partials = scr + recs*RT_SUMMARY_DOUBLES;
         unsigned int *tickets = (unsigned int *)(partials + g->n_tiles*RT_RED_SPLIT*RT_SUMMARY_DOUBLES);
-        const bool chunk_slots = g->chunks_per_tile <= g_last_grid;
+        /* with chunk slots the trace kernel wrote the sums into the records (grid_chunk_loop) */
+        const bool chunk_slots = g->chunks_per_tile <= grid;
         k_reduce_summary<<<(unsigned)(g->n_tiles*RT_RED_SPLIT), RT_RED_THREADS, 0, s>>>(
-            scr, recs/g->n_tiles, partials, tickets, summary,
-            (t->dynamic && !chunk_slots) ? scr + scratch_head_doubles(g) : nullptr, chunk_begin, chunk_end,
-            g->chunks_per_tile);
+            scr, recs/g->n_tiles, partials, tickets, summary, chunk_slots ? nullptr : item_sums,
+            chunk_begin, chunk_end, g->chunks_per_tile);
         g_launches++;
         CUDA_TRY(cudaGetLastError());
     }
