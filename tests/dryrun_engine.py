@@ -142,7 +142,7 @@ def trace_grid(table, grid, chunk_begin=0, chunk_end=None, outputs=E.GRID_OUTPUT
     r0, r1 = grid.first_ray_of_chunk(chunk_begin), grid.first_ray_of_chunk(chunk_end)
     spec = grid.c_spec()
     g = rt_oracle.trace_grid(spec, table.descs, table.n_by_wvl, r0, r1, opts, n_threads=4, wvls=table.wvls)
-    if full or (res is not None and res.full is not None):
+    if full or 'n_seg' in outputs or (res is not None and (res.full is not None or res.n_seg is not None)):
         p, d, wv, _ = rt_oracle.grid_start_rays(spec, r0, r1)
         b = rt_oracle.trace_bundle(table.descs, table.n_by_wvl, p, d, wv, opts, want_full=True,
                                    n_threads=4, wvls=table.wvls)

@@ -140,10 +140,31 @@ def test_grid_wavelength_rows_are_range_checked(tables):
     grid.close()
 
 
-@pytest.mark.parametrize('name,num', [('dblgauss', 64), ('rc', 50), ('cellphone', 33)])
+def spot_pieces_summary(spec, want, paths):
+    """the summary spot_diagram's pieces add up to, in the documented order (test_gpu_spot_sums):
+    rt_trace_grid_to_host splits the chunks at c0 + (c1 - c0)*i//n and adds the parts left to right.
+    ``paths``: record path of every piece whose path the launch size leaves open."""
+    from test_gpu_spot_sums import expected_summary, certain_paths, combine
+    nc = spec.n_chunks
+    n = min(max(1, min(8, nc//64)), nc)
+    parts = []
+    for i in range(n):
+        cb, ce = nc*i//n, nc*(i + 1)//n
+        a, b = spec.first_ray_of_chunk(cb), spec.first_ray_of_chunk(ce)
+        cand = certain_paths(spec, cb, ce)
+        parts.append(expected_summary(spec, cb, ce, want['abr'][:, a:b], want['op'][a:b],
+                                      want['status'][a:b], cand[0] if len(cand) == 1 else paths))
+    return combine(parts)
+
+
+@pytest.mark.parametrize('name,num', [('dblgauss', 64), ('rc', 50), ('cellphone', 33), ('dblgauss', 512)])
 def test_spot_diagram_end_to_end(tables, oracle, name, num):
     """analyses.spot_diagram (device chief rays, re-used grid block, 16 B/ray, pipelined copies):
-    aberrations / status / reference points equal the oracle's, twice in a row (grid re-use)."""
+    aberrations / status / reference points equal the oracle's, twice in a row (grid re-use); its
+    statistics are spot_statistics of the summary the pieces add up to in the documented order,
+    bit for bit, and lie within the rounding bound of a two-pass reference.  512^2: 8 pieces, tiles
+    crossing pieces."""
+    from test_gpu_spot_sums import DRYRUN, check_statistics
     opm, tab = tables(name)
     sm = opm.seq_model
     for rep in range(2):
@@ -168,6 +189,11 @@ def test_spot_diagram_end_to_end(tables, oracle, name, num):
                 m = ok[t*per:(t + 1)*per]
                 assert same(sd.grids[fi][wi], want['abr'][:, t*per:(t + 1)*per][:, m].T)
                 assert sd.summary['n_ok'][fi, wi] == m.sum()
+        got = {k: np.asarray(v).reshape(-1) for k, v in sd.summary.items()}
+        check_statistics(got, spec, want['abr'], want['op'], want['status'])
+        if not DRYRUN:
+            cands = [E.spot_statistics(spot_pieces_summary(spec, want, p)) for p in ('items', 'slots')]
+            assert any(all(same(got[k], c[k]) for k in got) for c in cands)
 
 
 @pytest.mark.parametrize('name', ['dblgauss', 'evenasph'])
